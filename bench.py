@@ -3,12 +3,13 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            this repo (one rank per GPU, torchrun for N > 1)
     python bench.py --impl reference [...]                         the reference's CPU path (rank 0 only)
+    python bench.py --dump-outputs DIR [...]                       also write the last timed step's outputs as DIR/<name>.npy
 
-Workload = BASELINE configs[2]: GenRe full_model inference, batch 16 per GPU, through the reference's FROZEN caller
-``models/genre_full_model.py:116-132 Net.forward`` (an unmodified copy staged in baseline/_ref) on top of this package's
-drop-in toolbox / networks: net1 (2D U-ResNet18, reference code on cuDNN) -> cam_bp -> render_spherical -> sph_pad ->
+Workload = BASELINE configs[2]: GenRe full_model inference, batch 16 per GPU, through
+``genre_shapehd_b200.genre_models.GenReNet.forward`` (the published models/genre_full_model.py:116-132 Net.forward) on this
+package's toolbox / networks: net1 (2D U-ResNet18 on cuDNN) -> cam_bp -> render_spherical -> sph_pad ->
 net2 (2D inpainting U-ResNet18) -> spherical back-projection -> Unet_3D refiner.  Random-init weights (no checkpoints
-offline; genre_shapehd_b200/synth_genre.py), synthetic rgb / silhouette inputs.  A "step" is one Net.forward over a batch.
+offline; genre_shapehd_b200/synth_genre.py), synthetic rgb / silhouette inputs.  A "step" is one forward over a batch.
 
 One JSON line on stdout (rank 0):
   value        whole-job shapes/s, inputs resident in HBM, device-timed, max over ranks
@@ -20,10 +21,10 @@ One JSON line on stdout (rank 0):
   cpu_baseline the reference arm (below) on a bounded sample, run as a sub-process on rank 0 at N = 1
   secondary    BASELINE configs[1] (cam_bp batch 32) and the same GenRe step with single-pass fp16 conv operands
   secondary_ddp  BASELINE configs[3] and [4]: ShapeHD fine-tune step and WGAN-GP critic step (batch 8 per GPU), GenRe end-to-end
-               fine-tune + Chamfer (batch 4 per GPU), frozen model classes, DDP over NCCL for N > 1 with the exposed all-reduce time
+               fine-tune + Chamfer (batch 4 per GPU), genre_shapehd_b200.genre_models classes, DDP over NCCL for N > 1 with the exposed all-reduce time
 
---impl reference: the same frozen Net.forward on the host CPU: toolbox ops = the CPU oracle port (the reference's ops are
-CUDA-only), networks = the reference's own networks/*.py on torch CPU, every host thread.
+--impl reference: the same GenReNet.forward on the host CPU: toolbox ops = the CPU oracle port (the reference's ops are
+CUDA-only), networks on torch CPU, every host thread.
 The oracle is only executed by that arm (and therefore by the cpu_baseline sub-process).
 """
 import argparse
@@ -48,6 +49,7 @@ FL, CAM_DIST = 418.3, 2.2
 METRIC = "GenRe shapes/sec @128^3 voxel (full_model inference); cam_bp HBM GB/s vs peak"
 UNIT = "shapes/s"
 UNET3D_GFLOP = 78.0          # per shape, forward (SURVEY 8a a12 / Appendix A)
+DUMP_BYTES = 60 << 20        # --dump-outputs: float32 payload of all arrays together (under 64 MB with the .npy headers)
 
 
 def parse():
@@ -62,12 +64,18 @@ def parse():
     ap.add_argument("--cpu-budget", type=float, default=150.0, help="--impl reference: wall-clock budget of the whole run (s)")
     ap.add_argument("--skip", default=os.environ.get("GENRE_B200_BENCH_SKIP", ""),
                     help="comma list of legs to skip: e2e,roofline,cpu,secondary,ddp")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float32, %d MiB in all: an "
+                         "output larger than its share of that as a fixed seeded sample" % (DUMP_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def config(args, n_gpus, extra=None):
     c = {"workload": "GenRe full_model inference (depth + sph-inpaint + voxel refine), batch=%d per GPU (BASELINE configs[2]), "
-                     "frozen models/genre_full_model.py Net.forward on the drop-in toolbox/networks" % args.batch,
+                     "GenReNet.forward (models/genre_full_model.py Net) on this package's toolbox/networks" % args.batch,
          "batch_per_gpu": args.batch, "global_batch": args.batch * n_gpus, "rgb_hw": [H, W], "voxel_res": RES,
          "weights": "random init (PyTorch defaults; min/max-depth head biased to the dataset depth range so cam_bp hits the grid)",
          "parallelism": "replicas x%d (batch-sharded, no collective)" % n_gpus,
@@ -128,7 +136,7 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------------------------------
-# reference arm: the frozen Net.forward on the host CPU (toolbox = oracle port, networks = the reference's own, torch CPU)
+# reference arm: GenReNet.forward on the host CPU (toolbox = oracle port, networks on torch CPU)
 # ----------------------------------------------------------------------------------------------------
 def _numa_node_cpus():
     """CPU sets of the host's NUMA nodes (within this process's affinity mask)"""
@@ -215,9 +223,8 @@ def run_reference(args):
             "warmup": warmup, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config(args, args.gpus),
             "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port",
-                             "sample": "%d of the %d shapes of a batch per step; frozen Net.forward on CPU: toolbox ops = oracle/genre_oracle.c "
-                                       "over a thread pool (the reference's ops are CUDA-only), 2D/3D networks = the reference's "
-                                       "networks/*.py on torch CPU; threads: %s (the faster of %d placements probed; host has %d logical CPUs)"
+                             "sample": "%d of the %d shapes of a batch per step; GenReNet.forward on CPU: toolbox ops = oracle/genre_oracle.c "
+                                       "over a thread pool (the reference's ops are CUDA-only), 2D/3D networks on torch CPU; threads: %s (the faster of %d placements probed; host has %d logical CPUs)"
                                        % (sample, args.batch, thread_desc, len(candidates), os.cpu_count() or 0)},
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0, "result_checksum": float(out.double().abs().sum())}
@@ -293,11 +300,11 @@ def graph_of(torch, fn, warm=2):
 def run_b200(args):
     import torch
 
-    from genre_shapehd_b200 import compat
-    compat.bootstrap()                       # frozen callers from baseline/_ref; toolbox / networks.networks from this package
-    from genre_shapehd_b200 import _lib, dist_util, ops_conv
-    from genre_shapehd_b200.synth_genre import genre_inputs, genre_opt, init_genre_net_for_bench
-    import models.genre_full_model as gfm
+    import genre_shapehd_b200
+    genre_shapehd_b200.install()
+    from genre_shapehd_b200 import _lib, compat, dist_util, ops_conv
+    from genre_shapehd_b200.genre_models import GenReNet
+    from genre_shapehd_b200.synth_genre import genre_inputs, init_genre_net_for_bench
 
     skip = set(x for x in args.skip.split(",") if x)
     world, rank, local = dist_util.env_world()
@@ -311,11 +318,11 @@ def run_b200(args):
 
     B, K, Wm = args.batch, args.steps, max(args.warmup, 3)
     torch.manual_seed(0)
-    net = gfm.Net(genre_opt(), gfm.Model)
+    net = GenReNet()
     init_genre_net_for_bench(net)
     net = net.to(dev).eval()
-    # the two 2D U-ResNet18 nets are the reference's own code (outside the hot path, SURVEY 8f-2); their one cheap win here is the
-    # memory format of the module instances (a deployment choice of the caller, no file of the reference is touched)
+    # the two 2D U-ResNet18 nets run on cuDNN (outside the hot path, SURVEY 8f-2); their one cheap win here is the
+    # memory format of the module instances
     nets2d = os.environ.get("GENRE_B200_BENCH_2D_FORMAT", "channels_last")
     if nets2d == "channels_last":
         net.depth_and_inpaint.net1.to(memory_format=torch.channels_last)
@@ -340,6 +347,10 @@ def run_b200(args):
         with torch.no_grad():
             return net(x)["pred_voxel"]
 
+    def forward_all(x):
+        with torch.no_grad():
+            return net(x)
+
     # launches of THIS library per step (eager, counted by the binding); cuDNN / aten kernels of the 2D nets are not ours
     forward(inputs[0])
     torch.cuda.synchronize()
@@ -353,17 +364,19 @@ def run_b200(args):
     if use_graph:
         try:
             for x in inputs:
-                replays.append(graph_of(torch, lambda x=x: forward(x)))
-        except Exception as e:       # e.g. an op of the frozen 2D nets that cannot be captured: launch from Python instead
+                replays.append(graph_of(torch, lambda x=x: forward_all(x)))
+        except Exception as e:       # e.g. an op of the 2D nets that cannot be captured: launch from Python instead
             graph_note = "capture failed: " + repr(e)[:160]
             use_graph, replays = False, []
             torch.cuda.synchronize()
 
     def step(i):
+        """one forward; returns the dict it computed (for a graph: the graph's output tensors, valid until its next replay)"""
         if use_graph:
-            replays[i % n_in][0]()
-        else:
-            forward(inputs[i % n_in])
+            replay, out = replays[i % n_in]
+            replay()
+            return out
+        return forward_all(inputs[i % n_in])
 
     for i in range(Wm):
         step(i)
@@ -380,7 +393,7 @@ def run_b200(args):
     t_wall0 = time.time()
     e0.record()
     for i in range(K):
-        step(i)
+        last = step(i)
     e1.record()
     barrier()
     t_wall1 = time.time()
@@ -388,6 +401,8 @@ def run_b200(args):
         torch.cuda.synchronize()
         torch.cuda.profiler.stop()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     t_load1 = t_wall1
     try:    # keep the same step running (untimed) so that nvidia-smi's 100 ms samples describe this kernel mix under load
         n_load = min(2000, max(K, int(0.6 / max(ms_total / K * 1e-3, 1e-6))))
@@ -450,13 +465,27 @@ def run_b200(args):
         line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": Wm,
                 "ms_per_step": ms_total / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "f32", "data": "synthetic",
-                "config": config(args, world, {"conv_mode": conv_mode, "nets2d": "reference uresnet.py modules on cuDNN (TF32 allowed, PyTorch default), %s" % nets2d}),
+                "config": config(args, world, {"conv_mode": conv_mode, "nets2d": "U-ResNet18 modules on cuDNN (TF32 allowed, PyTorch default), %s" % nets2d}),
                 "e2e": e2e, "gpu_launches": own_per_step * K,
                 "launch_mode": "cuda_graph" if use_graph else "python" + ("; " + graph_note if graph_note else ""),
                 "own_kernel_launches_per_step": own_per_step,
                 "roofline": roofline, "cpu_baseline": cpu, "clocks": clocks, "secondary": secondary, "secondary_ddp": ddp}
         print(json.dumps(line), flush=True)
     dist_util.finalize()
+
+
+def dump_outputs(out_dir, out):
+    """out: the dict of one GenReNet.forward.  Each tensor gets an equal share of DUMP_BYTES and is written as <name>.npy in
+    float32: whole when it fits its share, else the elements at that many sorted flat indices drawn from a generator
+    seeded with 0 (the same indices for the same shape in every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // (4 * len(out))
+    for name, t in sorted(out.items()):
+        a = t.detach().float().reshape(-1).cpu().numpy()
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.size != t.numel() else a.reshape(tuple(t.shape)))
 
 
 def e2e_leg(torch, net, dev, B, K, rank, world, barrier, max_over_ranks, use_graph, genre_inputs):

@@ -5,8 +5,8 @@ PyTorch on top of this package, without editing or copying them (SURVEY.md §7.1
     compat.bootstrap("/path/to/GenRe-ShapeHD")     # then: from models.genre_full_model import Net
 
 What it does:
-  * genre_shapehd_b200.install(reference_root): toolbox / nndistance / networks resolve HERE, everything else
-    (models, util, loggers, visualize, datasets, options, networks.uresnet/revresnet) in the reference checkout;
+  * genre_shapehd_b200.install(reference_root): toolbox / nndistance / networks.networks resolve HERE, everything
+    else (models, util, loggers, visualize, datasets, options, networks.uresnet/revresnet) in the reference checkout;
   * stubs the optional third-party modules the frozen files import at module level but never use on the
     differentiable path (skimage, trimesh; visualize/visualizer.py:8, util/util_sph.py:1-3);
   * makes torchvision's resnet18(pretrained=True) build offline (random init) — there is no network here.
@@ -39,18 +39,15 @@ def _unavailable(what):
 
 
 def find_reference():
-    """the frozen callers: $GENRE_REF, else the staged copy <repo>/baseline/_ref (travels to the GPU box), else /root/reference"""
-    for root in (os.environ.get("GENRE_REF"), os.path.join(genre_shapehd_b200.REPO_ROOT, "baseline", "_ref"), "/root/reference"):
-        if root and os.path.isdir(os.path.join(root, "models")):
-            return root
-    return None
+    """a checkout of the original GenRe-ShapeHD project named by $GENRE_REF, or None"""
+    root = os.environ.get("GENRE_REF")
+    return root if root and os.path.isdir(os.path.join(root, "models")) else None
 
 
 def bootstrap(reference_root=None, offline_resnet=True):
     root = reference_root or find_reference()
     if root is None or not os.path.isdir(os.path.join(root, "models")):
-        raise FileNotFoundError("no GenRe-ShapeHD checkout at %r (searched $GENRE_REF, <repo>/baseline/_ref, /root/reference; "
-                                "`python -c 'import __graft_entry__ as g; g.build()'` stages baseline/_ref)" % root)
+        raise FileNotFoundError("no GenRe-ShapeHD checkout at %r: pass its path or set $GENRE_REF" % root)
     os.environ["GENRE_REF"] = root
     genre_shapehd_b200.install(root)
     stub_optional_modules(offline_resnet)

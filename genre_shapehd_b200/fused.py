@@ -72,7 +72,7 @@ def genre_forward_fused(net, input_struct, glue=None):
     spherical map on the CPU through marching cubes + trimesh ray casting (util_sph.py:36-57), needs batch size 1 and is not
     differentiable: here the spherical map comes from the differentiable renderer, for any batch, on the device (SURVEY 8f-4).
 
-    net: models.genre_full_model.Net (reference class, unmodified), eval mode.  Returns the dict of Net.forward."""
+    net: genre_shapehd_b200.genre_models.GenReNet, eval mode.  Returns the dict of its forward."""
     dn = net.depth_and_inpaint
     if glue is None:
         glue = getattr(net, "_gb_glue", None)
@@ -80,7 +80,7 @@ def genre_forward_fused(net, input_struct, glue=None):
             glue = GenRe3DGlue(margin=net.margin).to(net.grid.device)
             net.__dict__["_gb_glue"] = glue
     out = dn.net1(input_struct)                                              # depth_pred_with_sph_inpaint.py:115-119
-    abs_depth = dn.get_abs_depth(out, input_struct)                         # :133-142 (frozen method)
+    abs_depth = dn.get_abs_depth(out, input_struct)                         # :133-142
     proj, sph_in = glue.project_and_render(abs_depth)                       # :120-126 cam_bp, clamp(proj * 50), render, sph_pad
     out_2 = dn.net2(sph_in)
     out["proj_depth"] = proj * glue.scale

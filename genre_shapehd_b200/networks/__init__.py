@@ -1,28 +1,10 @@
-"""Drop-in for the reference's ``networks`` package.
-
-``networks.networks`` (the 3D voxel nets, on the hot path) is provided here.  The 2D U-ResNet-18 modules
-(``networks.uresnet``, ``networks.revresnet``) are outside the hot path (SURVEY.md §2.1 #6) and keep resolving to a
-checkout of the reference when one is available: its ``networks`` directory is appended to this package's
-``__path__`` (nothing is copied).  Search order: $GENRE_REF, <repo>/baseline/_ref, /root/reference.
-"""
+"""Drop-in for the reference's ``networks`` package: ``networks.networks`` holds the 3D voxel nets (on the hot
+path).  The 2D U-ResNet-18s of GenRe are in genre_shapehd_b200/genre_models.py; genre_shapehd_b200.install() given a
+checkout of the reference appends its ``networks`` directory to this package's ``__path__``, so that the reference's
+own ``networks.uresnet`` / ``networks.revresnet`` resolve there (nothing is copied)."""
 import os
 import sys
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_REPO_ROOT = os.path.dirname(os.path.dirname(_HERE))
+_REPO_ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 if _REPO_ROOT not in sys.path:
     sys.path.append(_REPO_ROOT)
-
-
-def _reference_networks_dir():
-    for root in (os.environ.get("GENRE_REF"), os.path.join(_REPO_ROOT, "baseline", "_ref"), "/root/reference"):
-        if root:
-            d = os.path.join(root, "networks")
-            if os.path.isfile(os.path.join(d, "revresnet.py")):
-                return d
-    return None
-
-
-_ref = _reference_networks_dir()
-if _ref and _ref not in __path__:
-    __path__.append(_ref)

@@ -128,17 +128,13 @@ class ViewAsLinear(nn.Module):
 
 
 class ImageEncoder(nn.Module):
-    """2.5D sketch -> 200-d code (networks.py:6-22).  A 2D ResNet-18: outside the hot path, built from the
-    reference's own revresnet (resolved through this package's __path__, see networks/__init__.py)."""
+    """2.5D sketch -> 200-d code (networks.py:6-22).  A 2D ResNet-18 (torchvision's, randomly initialised): outside the
+    hot path."""
 
     def __init__(self, input_nc, encode_dims=200):
         super().__init__()
-        try:
-            from .revresnet import resnet18
-        except ImportError as e:
-            raise ImportError("ImageEncoder needs the reference's networks/revresnet.py (2D nets are out of scope "
-                              "here); set GENRE_REF to a GenRe-ShapeHD checkout") from e
-        resnet_m = resnet18(pretrained=True)
+        import torchvision
+        resnet_m = torchvision.models.resnet18(weights=None)
         resnet_m.conv1 = nn.Conv2d(input_nc, 64, 7, stride=2, padding=3, bias=False)
         resnet_m.avgpool = nn.AdaptiveAvgPool2d(1)
         resnet_m.fc = nn.Linear(512, encode_dims)

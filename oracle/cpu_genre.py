@@ -1,12 +1,12 @@
 """The reference's CPU path of the GenRe forward (BASELINE configs[2]) — BASELINE INFRASTRUCTURE, see cpu_toolbox/README.md.
 
-build_cpu_genre_net() returns the frozen models/genre_full_model.Net (the reference's file, from baseline/_ref or
-/root/reference) on CPU with
+build_cpu_genre_net() returns genre_shapehd_b200.genre_models.GenReNet (the published models/genre_full_model.Net) on CPU with
     toolbox.*            -> oracle/cpu_toolbox (the CUDA-only ops restated on the CPU oracle, maps in parallel)
-    networks.*           -> the reference's own networks/networks.py, uresnet.py, revresnet.py on torch CPU
+    networks.*           -> the 2D U-ResNets and networks/networks.py on torch CPU
 Must run in a process that never called genre_shapehd_b200.install() (bench.py --impl reference is such a process).
+
+    python oracle/cpu_genre.py        # one JSON line: forward_signatures() of that net
 """
-import argparse
 import os
 import sys
 
@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
 
 
-def build_cpu_genre_net(ref_root=None):
+def build_cpu_genre_net():
     import torch
     for name in ("toolbox", "networks", "nndistance"):
         if name in sys.modules:
@@ -22,21 +22,39 @@ def build_cpu_genre_net(ref_root=None):
                                % (name, getattr(sys.modules[name], "__file__", "?")))
     if REPO not in sys.path:
         sys.path.insert(0, REPO)
-    from genre_shapehd_b200 import compat
-    from genre_shapehd_b200.synth_genre import init_genre_net_for_bench
-    ref_root = ref_root or compat.find_reference()
-    if ref_root is None:
-        raise FileNotFoundError("no staged reference callers (baseline/_ref): run __graft_entry__.build() where /root/reference exists")
-    sys.path.insert(0, ref_root)                                    # models, util, networks (the reference's own, CPU torch)
+    sys.path.insert(0, os.path.join(REPO, "genre_shapehd_b200"))     # networks
     sys.path.insert(0, os.path.join(HERE, "cpu_toolbox"))           # toolbox -> CPU oracle stand-ins
-    compat.stub_optional_modules()
-    import models.genre_full_model as gfm
+    from genre_shapehd_b200.genre_models import GenReNet
+    from genre_shapehd_b200.synth_genre import init_genre_net_for_bench
     import toolbox
     assert os.path.abspath(toolbox.__file__).startswith(os.path.join(HERE, "cpu_toolbox"))
-    assert os.path.abspath(gfm.Unet_3D.__module__ and sys.modules[gfm.Unet_3D.__module__].__file__).startswith(os.path.abspath(ref_root))
-    opt = argparse.Namespace(joint_train=False, padding_margin=16, inpaint_path=None, pred_depth_minmax=True,
-                             net1_path=None, load_offline=False)
     torch.manual_seed(0)
-    net = gfm.Net(opt, gfm.Model)
+    net = GenReNet()
     init_genre_net_for_bench(net)
     return net.eval()
+
+
+FORWARD_BATCH, FORWARD_SEED, FORWARD_THREADS = 1, 0, 4
+
+
+def forward_signatures(net, n=64):
+    """eval forward of a GenRe net on genre_inputs(FORWARD_BATCH, seed=FORWARD_SEED), FORWARD_THREADS torch threads:
+    for every output, its shape, float64 sum and |sum| and n values at evenly spaced flat indices"""
+    import torch
+    from genre_shapehd_b200.synth_genre import genre_inputs
+    torch.set_num_threads(FORWARD_THREADS)
+    with torch.no_grad():
+        out = net(genre_inputs(FORWARD_BATCH, seed=FORWARD_SEED))
+    sig = {}
+    for k, t in out.items():
+        flat = t.detach().reshape(-1).double()
+        idx = torch.linspace(0, flat.numel() - 1, n).long()
+        sig[k] = {"shape": list(t.shape), "sum": float(flat.sum()), "abs_sum": float(flat.abs().sum()),
+                  "samples": [float(v) for v in flat[idx]]}
+    return sig
+
+
+if __name__ == "__main__":
+    import json
+    sys.path[:] = [p for p in sys.path if os.path.abspath(p or ".") != HERE]     # `oracle` is the package, not oracle.py
+    print(json.dumps(forward_signatures(build_cpu_genre_net())))

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """BASELINE configs[3] and [4] (ShapeHD fine-tune step and 3D-WGAN-GP critic step, batch 8 per GPU; GenRe end-to-end fine-tune
 with the Chamfer op, batch 4 per GPU; DDP over NCCL) on the
-networks drop-in, driven through the reference's FROZEN classes (baseline/_ref):
+networks drop-in, driven through genre_shapehd_b200.genre_models (the published model classes):
   shapehd step : models/shapehd.py Net (:82-118: two marrnet2 = ImageEncoder -> VoxelDecoder, frozen D) + the loss of
                  :67-79 (BCE-with-logits + w * -mean(D(sigmoid(voxel)))) + Adam on marrnet2 (:42-47)
   wgangp D step: models/wgangp.py:77-112,144-164 restated on its own D / G classes (:193-214): D(real), D(G(z)) and the
@@ -29,17 +29,16 @@ if REPO not in sys.path:
 
 
 def run(dev, world, rank, local, batch=8, steps=6, warmup=3, which=("shapehd", "wgan", "genre"), genre_batch=4):
-    from genre_shapehd_b200 import compat, dist_util, ops_conv
-    compat.bootstrap()
-    import models.shapehd as shd
-    import models.wgangp as wg
+    import genre_shapehd_b200
+    genre_shapehd_b200.install()
+    from genre_shapehd_b200 import dist_util, genre_models, ops_conv
     from torch.nn.parallel import DistributedDataParallel as DDP
 
     torch.manual_seed(1 + rank)
     B = batch
     res = {"n_gpus": world, "batch_per_gpu": B, "steps": steps, "conv_mode": ops_conv.describe_mode(),
            "bn_train_custom": ops_conv.BN_TRAIN, "tc_backward": ops_conv.TC_BACKWARD,
-           "workload": "BASELINE configs[3]: frozen models/shapehd.py Net + loss, and models/wgangp.py critic step, DDP over NCCL"}
+           "workload": "BASELINE configs[3]: ShapeHDNet (models/shapehd.py Net) + loss, and the models/wgangp.py critic step, DDP over NCCL"}
 
     def wrap(m):
         return DDP(m, device_ids=[local], gradient_as_bucket_view=True) if world > 1 else m
@@ -61,7 +60,7 @@ def run(dev, world, rank, local, batch=8, steps=6, warmup=3, which=("shapehd", "
 
     # ---- ShapeHD fine-tune step ---------------------------------------------------------------------------------------
     if "shapehd" in which:
-        net = shd.Net().to(dev)
+        net = genre_models.ShapeHDNet().to(dev)
         net.train()
         ddp = wrap(net)
         opt = torch.optim.Adam(net.marrnet2.parameters(), lr=1e-3)
@@ -90,9 +89,8 @@ def run(dev, world, rank, local, batch=8, steps=6, warmup=3, which=("shapehd", "
 
     # ---- WGAN-GP critic step ---------------------------------------------------------------------------------------------
     if "wgan" in which:
-        G = wg.G(200).to(dev)
-        G.noise = G.noise.to(dev)
-        Dn = wg.D().to(dev)
+        G = genre_models.WganGenerator(200).to(dev)
+        Dn = genre_models.WganCritic().to(dev)
         for p in G.parameters():
             p.requires_grad = False
         ddp_d = wrap(Dn)
@@ -129,11 +127,10 @@ def run(dev, world, rank, local, batch=8, steps=6, warmup=3, which=("shapehd", "
                                          "allreduce_bytes": 4 * sum(p.numel() for p in Dn.parameters())})
     # ---- GenRe end-to-end fine-tune step + Chamfer (BASELINE configs[4], batch 4 per GPU) ---------------------------------
     if "genre" in which:
-        import models.genre_full_model as gfm
-        from genre_shapehd_b200.synth_genre import genre_inputs, genre_opt, init_genre_net_for_bench
+        from genre_shapehd_b200.synth_genre import genre_inputs, init_genre_net_for_bench
         from nndistance.functions.nnd import nndistance
         Bg = genre_batch
-        gnet = gfm.Net(genre_opt(joint_train=True), gfm.Model)       # frozen class; joint_train: gradients reach net1 / net2
+        gnet = genre_models.GenReNet(joint_train=True)                # joint_train: gradients reach net1 / net2
         init_genre_net_for_bench(gnet)                                # through cam_bp / render_spherical / spherical bp backward
         gnet = gnet.to(dev).train()
         gddp = wrap(gnet)
@@ -167,7 +164,7 @@ def run(dev, world, rank, local, batch=8, steps=6, warmup=3, which=("shapehd", "
         ms, loss = timed(genre_step)
         res["genre_finetune"] = {"batch_per_gpu": Bg, "step_ms": ms, "shapes_per_s": world * Bg / ms * 1e3, "loss_finite": bool(loss == loss),
                                  "chamfer_points": npts,
-                                 "workload": "BASELINE configs[4]: frozen genre_full_model.Net, joint_train, voxel + surface loss, "
+                                 "workload": "BASELINE configs[4]: GenReNet, joint_train, voxel + surface loss, "
                                              "backward through every toolbox op, + nndistance fwd/bwd on [B,4096,3] clouds"}
         if world > 1:
             ms_ns, _ = timed(lambda: genre_step(sync=False))

@@ -1,20 +1,20 @@
 #!/usr/bin/env python
-"""Where the GenRe full-model forward (BASELINE configs[2], batch 16, frozen Net.forward on the drop-in) spends its time:
+"""Where the GenRe full-model forward (BASELINE configs[2], batch 16, GenReNet.forward) spends its time:
 CUDA events around the sub-modules (forward hooks, eager launches), and the effect of the 2D nets' "cheap wins"
 (channels_last; bf16 autocast) on the whole step.  One JSON line."""
 import json, os, sys
 import torch
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, REPO)
-from genre_shapehd_b200 import compat
-compat.bootstrap()
+import genre_shapehd_b200
+genre_shapehd_b200.install()
 from genre_shapehd_b200 import ops_conv
-from genre_shapehd_b200.synth_genre import genre_inputs, genre_opt, init_genre_net_for_bench
-import models.genre_full_model as gfm
+from genre_shapehd_b200.genre_models import GenReNet
+from genre_shapehd_b200.synth_genre import genre_inputs, init_genre_net_for_bench
 dev = torch.device("cuda:0"); torch.cuda.set_device(dev)
 B = int(os.environ.get("B", 16))
 torch.manual_seed(0)
-net = gfm.Net(genre_opt(), gfm.Model); init_genre_net_for_bench(net); net = net.to(dev).eval()
+net = GenReNet(); init_genre_net_for_bench(net); net = net.to(dev).eval()
 x = genre_inputs(B, dev, seed=0)
 
 def timeit(fn, reps=10, warm=3):

@@ -1,10 +1,14 @@
 """GPU parity tests: the CUDA path, called through the C ABI (via the Python mirror of the reference's
 toolbox packages), against
   (1) the CPU oracle (oracle/genre_oracle.c) on seeded inputs small enough to finish in seconds,
-  (2) the reference's OWN kernels compiled unmodified into oracle/_ref (oracle/ref_gpu.py), at BASELINE sizes,
+  (2) the reference's OWN kernels at BASELINE sizes, through golden outputs recorded from them
+      (tests/golden/ref_*.npz, written by tests/golden/make_golden_fullsize.py),
   (3) size-independent properties (point conservation, determinism, idempotence).
 Bars (BASELINE.json north_star): voxel / neighbour indices bit-exact, values within 1e-4 (most are far tighter).
 """
+import hashlib
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -12,7 +16,6 @@ import torch
 from genre_shapehd_b200 import _lib
 from genre_shapehd_b200.synth import sphere_depth, uniform_depth
 from nndistance.functions.nnd import NNDFunction, nndistance, nndistance_score
-from oracle import ref_gpu
 from toolbox.calc_prob.calc_prob.functions.calc_prob import CalcStopProb
 from toolbox.cam_bp.cam_bp._ext import cam_bp_lib
 from toolbox.cam_bp.cam_bp.functions import CameraBackProjection, SphericalBackProjection, get_surface_mask
@@ -21,7 +24,31 @@ from toolbox.spherical_proj import gen_sph_grid, render_spherical, sph_pad
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-needs_ref = pytest.mark.skipif(not ref_gpu.available(), reason="oracle/_ref reference kernels not built")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def golden(name):
+    """outputs of the reference's own kernels on the test's inputs (see tests/golden/make_golden_fullsize.py)"""
+    return np.load(os.path.join(GOLDEN, name + ".npz"))
+
+
+def sha(t):
+    return hashlib.sha256(t.detach().contiguous().cpu().numpy().tobytes()).hexdigest()
+
+
+def assert_sampled(got, r, name, tol, stride):
+    """|got - reference| <= tol at the stored every-stride-th elements, and over the whole tensor on average"""
+    flat = got.detach().reshape(-1)
+    assert (flat[::stride].cpu() - torch.from_numpy(r[name])).abs().max().item() <= tol, name
+    assert abs(flat.double().sum().item() - float(r[name + "_sum_f64"])) <= tol * flat.numel(), name
+
+
+def assert_hits(tdf, cnt, r, tol):
+    """a back-projection against the reference's: counts bit for bit, distances at every stored hit voxel"""
+    assert sha(cnt) == str(r["cnt_sha256"]), "counts differ from the reference kernel"
+    idx = torch.from_numpy(r["idx"].astype(np.int64)).to(tdf.device)
+    assert (tdf.reshape(-1)[idx].cpu() - torch.from_numpy(r["tdf"])).abs().max().item() < tol
+    assert abs(tdf.double().sum().item() - float(r["tdf_sum_f64"])) <= tol * tdf.numel()
 
 
 def dev(a, dtype=torch.float32):
@@ -129,25 +156,24 @@ def test_cam_bp_forward_bucket_overflow_wall(oracle):
     assert per_tile.max() > 1024
 
 
-@needs_ref
 @pytest.mark.parametrize("n", [1, 4])
 def test_cam_bp_forward_vs_reference_kernel_at_full_size(oracle, n):
+    r = golden("ref_cam_bp_forward_n%d" % n)
     d = oracle.bench_depth_batch(n)
     depth = dev(d)
     fl = torch.full((n, 1), 418.3, device=DEV)
     cd = torch.full((n, 1), 2.2, device=DEV)
-    tdf_r, cnt_r = ref_gpu.cam_bp_forward(depth, fl, cd, 128)
-    tdf = torch.empty_like(tdf_r)
-    cnt = torch.empty_like(tdf_r)
+    tdf = torch.empty((n, 1, 128, 128, 128), device=DEV)
+    cnt = torch.empty_like(tdf)
     cam_bp_lib.back_projection_forward(depth, cd, fl, tdf, cnt)
-    assert torch.equal(cnt, cnt_r), "counts differ from the reference kernel"
-    assert (cnt.sum().item()) > 10000 * n
-    assert (tdf - tdf_r).abs().max().item() < 1e-7
+    assert_hits(tdf, cnt, r, 1e-7)
+    assert (cnt.sum().item()) > 10000 * n and int((cnt != 0).sum()) == int(r["n_hits"])
     # module path with fused shift == reference module path (shift_tdf as two dense torch ops)
     out = Camera_back_projection_layer()(depth)
-    ref_out = 1 - 128 * tdf_r
-    assert (out - ref_out).abs().max().item() < 1e-5
-    assert torch.equal(out == 0, cnt_r == 0)
+    idx = torch.from_numpy(r["idx"].astype(np.int64)).to(DEV)
+    assert (out.reshape(-1)[idx].cpu() - (1 - 128 * torch.from_numpy(r["tdf"]))).abs().max().item() < 1e-5
+    assert (out - (1 - 128 * tdf)).abs().max().item() < 1e-5
+    assert torch.equal(out == 0, cnt == 0)
 
 
 def test_cam_bp_forward_is_bitwise_deterministic(oracle):
@@ -192,22 +218,25 @@ def test_cam_bp_backward_vs_oracle(oracle, res, hw, n, c):
         np.testing.assert_allclose(depth2.grad.cpu().numpy(), -128 * gd_o, atol=2e-3, rtol=1e-4)
 
 
-@needs_ref
 def test_cam_bp_backward_vs_reference_kernel_single_sample(oracle):
     """N == 1 only: the reference kernel reads cam_dist out of bounds for n >= 1 (back_projection_kernel.cu:401)."""
+    r = golden("ref_cam_bp_backward")
     d = dev(oracle.bench_depth_batch(2)[1:2])
     fl = torch.full((1, 1), 418.3, device=DEV)
     cd = torch.full((1, 1), 2.2, device=DEV)
-    _, cnt = ref_gpu.cam_bp_forward(d, fl, cd, 128)
+    tdf = torch.empty((1, 1, 128, 128, 128), device=DEV)
+    cnt = torch.empty_like(tdf)
+    cam_bp_lib.back_projection_forward(d, cd, fl, tdf, cnt)
+    assert_hits(tdf, cnt, r, 1e-7)
     g = torch.randn(1, 1, 128, 128, 128, device=DEV, generator=torch.Generator(DEV).manual_seed(0))
-    gd_r, gfl_r, gcd_r = ref_gpu.cam_bp_backward(d, fl, cd, cnt, g)
-    gd = torch.empty_like(gd_r)
-    gfl = torch.empty_like(gfl_r)
-    gcd = torch.empty_like(gcd_r)
+    gfl_r, gcd_r = float(r["grad_fl"].reshape(-1)[0]), float(r["grad_camdist"].reshape(-1)[0])
+    gd = torch.empty_like(d)
+    gfl = torch.empty(r["grad_fl"].shape, device=DEV)
+    gcd = torch.empty(r["grad_camdist"].shape, device=DEV)
     cam_bp_lib.back_projection_backward(d, fl, cd, cnt, g, gd, gcd, gfl)
-    assert (gd - gd_r).abs().max().item() < 1e-5
-    assert abs(gfl.item() - gfl_r.item()) <= 2e-4 * max(1.0, abs(gfl_r.item()))
-    assert abs(gcd.item() - gcd_r.item()) <= 2e-4 * max(1.0, abs(gcd_r.item()))
+    assert_sampled(gd, r, "grad_depth", 1e-5, 14)
+    assert abs(gfl.item() - gfl_r) <= 2e-4 * max(1.0, abs(gfl_r))
+    assert abs(gcd.item() - gcd_r) <= 2e-4 * max(1.0, abs(gcd_r))
 
 
 @pytest.mark.parametrize("res,hw", [(32, 64), (21, 40)])
@@ -222,18 +251,20 @@ def test_surface_mask_vs_oracle(oracle, res, hw):
     assert np.array_equal(surf.cpu().numpy(), np.clip(cnt_o, 0, 1))
 
 
-@needs_ref
 def test_surface_mask_vs_reference_kernel(oracle):
+    r = golden("ref_surface_mask")
     d = oracle.bench_depth_batch(2)
     d[d == 0] = -1.0
     depth = dev(d)
     fl = torch.full((2, 1), 418.3, device=DEV)
     cd = torch.full((2, 1), 2.2, device=DEV)
-    _, cnt = ref_gpu.cam_bp_forward(depth, fl, cd, 128)
-    mask_r = ref_gpu.surface_mask(depth, fl, cd, cnt)
-    mask = torch.empty_like(mask_r)
+    tdf = torch.empty((2, 1, 128, 128, 128), device=DEV)
+    cnt = torch.empty_like(tdf)
+    cam_bp_lib.back_projection_forward(depth, cd, fl, tdf, cnt)
+    assert sha(cnt) == str(r["cnt_sha256"])
+    mask = torch.empty_like(cnt)
     cam_bp_lib.get_surface_mask(depth, cd, fl, cnt, mask)
-    assert torch.equal(mask, mask_r)
+    assert sha(mask) == str(r["mask_sha256"]), "surface mask differs from the reference kernel"
     assert 0.05 < (mask == 0).float().mean().item() < 0.9
 
 
@@ -266,22 +297,19 @@ def test_sph_bp_forward_backward_vs_oracle(oracle, res, s, n):
     np.testing.assert_allclose(x.grad.cpu().numpy(), gs_o, atol=2e-4 * max(1.0, np.abs(gs_o).max()), rtol=2e-3)
 
 
-@needs_ref
 def test_sph_bp_vs_reference_kernels_full_size():
+    r = golden("ref_sph_bp")
     n = 3
     sph = dev(_sph_inputs(n, 128, 5))
     grid = gen_sph_grid().to(DEV).expand(n, -1, -1, -1, -1)
-    tdf_r, cnt_r = ref_gpu.sph_bp_forward(sph, grid, 128)
-    tdf = torch.empty_like(tdf_r)
-    cnt = torch.empty_like(tdf_r)
+    tdf = torch.empty((n, 1, 128, 128, 128), device=DEV)
+    cnt = torch.empty_like(tdf)
     cam_bp_lib.spherical_back_proj_forward(sph, grid, tdf, cnt)
-    assert torch.equal(cnt, cnt_r)
-    assert (tdf - tdf_r).abs().max().item() < 1e-7
+    assert_hits(tdf, cnt, r, 1e-7)
     g = torch.randn(tdf.shape, device=DEV, generator=torch.Generator(DEV).manual_seed(1))
-    gs_r = ref_gpu.sph_bp_backward(sph, grid, cnt_r, g)
-    gs = torch.empty_like(gs_r)
+    gs = torch.empty_like(sph)
     cam_bp_lib.spherical_back_proj_backward(sph, grid, cnt, g, gs)
-    assert (gs - gs_r).abs().max().item() <= 1e-4 * max(1.0, gs_r.abs().max().item())
+    assert_sampled(gs, r, "grad_sph", 1e-4 * max(1.0, float(r["grad_sph_absmax"])), 14)
 
 
 def test_genre_backproject_spherical_glue_runs_on_the_new_op():
@@ -316,7 +344,6 @@ def test_calc_prob_vs_oracle(oracle, shape):
     np.testing.assert_allclose(x.grad.cpu().numpy(), grad_o, rtol=1e-3, atol=1e-5 * scale)
 
 
-@needs_ref
 def test_calc_prob_backward_is_finite_when_the_last_sample_is_certain():
     """ADVICE r1: p[Z-1] == 1 made the last sample's gradient 0/0; the reference special-cases it as w/p (calc_prob_kernel.cu:169-172)"""
     p = torch.rand(3, 1, 4, 4, 64, device=DEV).clamp_(0.05, 0.95)
@@ -331,20 +358,27 @@ def test_calc_prob_backward_is_finite_when_the_last_sample_is_certain():
     assert torch.allclose(gp[..., -1], g[..., -1] * trans, rtol=1e-4, atol=1e-7)
 
 
-def test_calc_prob_vs_reference_kernels_full_size():
+def test_calc_prob_vs_reference_kernels_full_size(oracle):
+    """every element against the CPU oracle (the reference's loop order, one rounding per fp32 op), and a fixed subset of
+    the elements against the reference's own kernels"""
     gen = torch.Generator(DEV).manual_seed(0)
     p = torch.rand(2, 1, 128, 128, 256, device=DEV, generator=gen).clamp_(1e-5, 1 - 1e-5)
     p = torch.where(torch.rand(p.shape, device=DEV, generator=gen) < 0.9, torch.full_like(p, 1e-5), p)
-    s_r = ref_gpu.calc_prob_forward(p)
+    r = golden("ref_calc_prob")
+    k = int(r["stride"])
     s = CalcStopProb.apply(p)
-    assert (s - s_r).abs().max().item() < 1e-5
-    torch.testing.assert_close(s, s_r, rtol=1e-4, atol=1e-7)
+    s_o = torch.from_numpy(oracle.calc_prob_forward(p.cpu().numpy()))
+    assert (s.cpu() - s_o).abs().max().item() < 1e-5
+    torch.testing.assert_close(s.cpu(), s_o, rtol=1e-4, atol=1e-7)
+    assert_sampled(s, r, "stop", 1e-5, k)
+    torch.testing.assert_close(s.reshape(-1)[::k].cpu(), torch.from_numpy(r["stop"]), rtol=1e-4, atol=1e-7)
     g = torch.randn(p.shape, device=DEV, generator=gen)
-    gr_r = ref_gpu.calc_prob_backward(p, s_r * g)
     from toolbox.calc_prob.calc_prob._ext import calc_prob_lib
     gr = torch.empty_like(p)
-    calc_prob_lib.calc_prob_backward(p, (s_r * g).contiguous(), gr)
-    assert (gr - gr_r).abs().max().item() <= 1e-4 * gr_r.abs().max().item()
+    calc_prob_lib.calc_prob_backward(p, (s * g).contiguous(), gr)
+    gr_o = torch.from_numpy(oracle.calc_prob_backward(p.cpu().numpy(), (s * g).cpu().numpy()))
+    assert (gr.cpu() - gr_o).abs().max().item() <= 1e-4 * gr_o.abs().max().item()
+    assert_sampled(gr, r, "grad_prob", 1e-4 * float(r["grad_prob_absmax"]), k)
 
 
 # --------------------------------------------------------------------------------------------------
@@ -496,22 +530,21 @@ def test_nnd_forward_backward_vs_oracle(oracle, b, n, m):
     np.testing.assert_allclose(x2.grad.cpu().numpy(), o2, atol=1e-5)
 
 
-@needs_ref
 @pytest.mark.parametrize("b,n,m", [(4, 4096, 4096), (2, 3000, 5000)])
 def test_nnd_vs_reference_kernels(b, n, m):
+    r = golden("ref_nnd_%d_%d_%d" % (b, n, m))
     gen = torch.Generator(DEV).manual_seed(n)
     x1 = torch.rand(b, n, 3, device=DEV, generator=gen) - 0.5
     x2 = torch.rand(b, m, 3, device=DEV, generator=gen) - 0.5
-    d1r, d2r, i1r, i2r = ref_gpu.nnd_forward(x1, x2)
     d1, d2, i1, i2 = NNDFunction.apply(x1, x2)
-    assert torch.equal(i1, i1r) and torch.equal(i2, i2r)
-    assert torch.equal(d1, d1r) and torch.equal(d2, d2r)
+    assert sha(i1) == str(r["idx1_sha256"]) and sha(i2) == str(r["idx2_sha256"])
+    assert sha(d1) == str(r["dist1_sha256"]) and sha(d2) == str(r["dist2_sha256"])
     g1, g2 = torch.rand(b, n, device=DEV, generator=gen), torch.rand(b, m, device=DEV, generator=gen)
-    o1r, o2r = ref_gpu.nnd_backward(x1, x2, g1, g2, i1r, i2r)
     from nndistance._ext import my_lib
     o1, o2 = torch.empty_like(x1), torch.empty_like(x2)
     my_lib.nnd_backward_cuda(x1, x2, o1, o2, g1, g2, i1, i2)
-    assert (o1 - o1r).abs().max().item() < 1e-5 and (o2 - o2r).abs().max().item() < 1e-5
+    assert_sampled(o1, r, "grad_xyz1", 1e-5, 14)
+    assert_sampled(o2, r, "grad_xyz2", 1e-5, 14)
 
 
 def test_nnd_score_and_layouts():

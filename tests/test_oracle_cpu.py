@@ -1,7 +1,9 @@
 """CPU-only checks of the oracle (oracle/genre_oracle.c): against the reference's own CPU code where it has
-any (nndistance, my_lib.c compiled unmodified), against independent float64 restatements, against the
+any (nndistance, my_lib.c: its outputs stored in tests/golden/ref_nnd_cpu.npz), against independent float64 restatements, against the
 torch-CPU composition the reference's render_spherical is written in, and the C1 plumbing config
 (depth -> voxel -> spherical on one 256x256 map, SURVEY.md §8d)."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -13,13 +15,12 @@ from toolbox.spherical_proj import gen_sph_grid, render_spherical
 # nndistance: the only op with a CPU implementation in the reference
 # --------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("b,n,m,seed", [(1, 50, 50, 0), (2, 257, 129, 1), (3, 64, 700, 2)])
-def test_nnd_oracle_matches_reference_cpu_code(oracle, b, n, m, seed):
-    if not oracle.ref_available("libref_nnd_cpu.so"):
-        pytest.skip("oracle/_ref/libref_nnd_cpu.so not built")
+def test_nnd_oracle_matches_reference_cpu_code(oracle, golden_dir, b, n, m, seed):
     rng = np.random.RandomState(seed)
     p1 = (rng.rand(b, n, 3) * 20).astype(np.float32)  # the reference demo's scale (nndistance/test.py:11-12)
     p2 = (rng.rand(b, m, 3) * 20).astype(np.float32)
-    d_ref, i_ref = oracle.ref_nnsearch_cpu(p1, p2)
+    ref = np.load(os.path.join(golden_dir, "ref_nnd_cpu.npz"))     # tests/golden/make_golden_fullsize.py
+    d_ref, i_ref = ref["dist_%d" % seed], ref["idx_%d" % seed]
     d, i = oracle.nnsearch(p1, p2, fused=False)
     assert np.array_equal(i, i_ref)
     assert np.array_equal(d, d_ref)
