@@ -11,8 +11,6 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libgenre_b200.so")
 
 FLAG_SHIFT_TDF = 1
-FLAG_OVERLAP = 2   # cam_bp_forward, experimental: project and splat overlapped in one kernel (GENRE_B200_CAM_BP_OVERLAP=1); measured slower
-CAM_BP_FLAGS = FLAG_OVERLAP if os.environ.get("GENRE_B200_CAM_BP_OVERLAP", "0") != "0" else 0
 
 _i64 = ctypes.c_int64
 _int = ctypes.c_int
@@ -81,7 +79,7 @@ EXPORTED_SYMBOLS = sorted(list(_SIGNATURES) + [
     "genre_b200_last_error", "genre_b200_version", "genre_b200_voxelize_workspace_bytes",
     "genre_b200_convt_c1_wgrad_workspace_bytes", "genre_b200_conv_k8s2_wgrad_workspace_bytes",
     "genre_b200_bn_workspace_bytes", "genre_b200_render_spherical_workspace_bytes",
-    "genre_b200_voxel_surface_workspace_bytes", "genre_b200_conv_set_tma", "genre_b200_conv_set_cluster", "genre_b200_convflat_positions", "genre_b200_skinny_gemm_workspace_bytes"])
+    "genre_b200_voxel_surface_workspace_bytes", "genre_b200_convflat_positions", "genre_b200_skinny_gemm_workspace_bytes"])
 
 _lib = None
 launch_count = 0  # kernels of this library enqueued through the binding (bench.py reports it as gpu_launches)
@@ -129,10 +127,6 @@ def load():
     lib.genre_b200_bn_workspace_bytes.argtypes = [_i64]
     lib.genre_b200_render_spherical_workspace_bytes.restype = _size
     lib.genre_b200_render_spherical_workspace_bytes.argtypes = [_i64, _int]
-    lib.genre_b200_conv_set_tma.restype = _int
-    lib.genre_b200_conv_set_tma.argtypes = [_int]
-    lib.genre_b200_conv_set_cluster.restype = _int
-    lib.genre_b200_conv_set_cluster.argtypes = [_int]
     lib.genre_b200_skinny_gemm_workspace_bytes.restype = _size
     lib.genre_b200_skinny_gemm_workspace_bytes.argtypes = [_i64, _i64, _i64, _int]
     lib.genre_b200_convflat_positions.restype = _i64

@@ -155,14 +155,6 @@ cam_project_kernel(const CamProjArgs a) {
   cam_project_body<W_FAST>(a, blockIdx.x, blockIdx.y, s_hist);
 }
 
-template <bool W_FAST>
-struct CamProjector {   // project stage of the overlapped kernel (voxelize.cuh vox_overlap_kernel)
-  using Args = CamProjArgs;
-  static __device__ __forceinline__ void run(const Args &a, int bx, int map, unsigned *s_hist) {
-    cam_project_body<W_FAST>(a, bx, map, s_hist);
-  }
-};
-
 static int cam_check(const float *depth, int64_t N, int64_t C, int64_t H, int64_t W, const float *fl,
                      const float *camdist, int res) {
   GB_REQUIRE(depth && fl && camdist, GENRE_B200_EINVAL, "cam_bp: null input pointer");
@@ -377,6 +369,8 @@ extern "C" int genre_b200_cam_bp_forward(const float *depth, int64_t N, int64_t 
                                          unsigned flags, void *workspace, size_t workspace_bytes, void *stream) {
   if (int rc = cam_check(depth, N, C, H, W, fl, camdist, res)) return rc;
   GB_REQUIRE(tdf != nullptr, GENRE_B200_EINVAL, "cam_bp: tdf is null");
+  GB_REQUIRE((flags & ~(unsigned)GENRE_B200_FLAG_SHIFT_TDF) == 0, GENRE_B200_EINVAL,
+             "cam_bp: unknown flag bits 0x%x (only GENRE_B200_FLAG_SHIFT_TDF = 1 is defined)", flags & ~(unsigned)GENRE_B200_FLAG_SHIFT_TDF);
   VoxWorkspace w;
   GB_REQUIRE(vox_carve(workspace, workspace_bytes, N * C, H * W, res, &w), GENRE_B200_EWORKSPACE,
              "cam_bp: workspace too small or misaligned (need %zu bytes)", vox_workspace_bytes(N * C, H * W, res));
@@ -396,17 +390,6 @@ extern "C" int genre_b200_cam_bp_forward(const float *depth, int64_t N, int64_t 
     bg = inv_r;
   }
   if (int rc = vox_clear_counts(w, N * C, st)) return rc;
-  if (flags & GENRE_B200_FLAG_OVERLAP) {
-    // experimental, off by default (measured slower): project and splat in ONE kernel with an interleaved block order
-    // (voxelize.cuh vox_overlap_kernel)
-    CamProjArgs a;
-    bool w_fast = true;
-    if (int rc = cam_proj_args(depth, N, C, H, W, sN, sC, sH, sW, fl, fN, fC, camdist, dN, dC, res, w, &a, &w_fast)) return rc;
-    const int gx = cam_proj_ctas_per_map(H * W);
-    const int rc = w_fast ? vox_overlap<CamProjector<true>>(a, gx, w, N * C, H * W, res, tdf, cnt, alpha, beta, bg, st)
-                          : vox_overlap<CamProjector<false>>(a, gx, w, N * C, H * W, res, tdf, cnt, alpha, beta, bg, st);
-    if (rc >= 0) return rc;
-  }
   if (int rc = cam_project_launch(depth, N, C, H, W, sN, sC, sH, sW, fl, fN, fC, camdist, dN, dC, res, w, st)) return rc;
   return vox_splat(w, N * C, H * W, res, tdf, cnt, alpha, beta, bg, st);
 }

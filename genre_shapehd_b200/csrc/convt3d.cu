@@ -17,11 +17,10 @@
 // K-chunk) stage and arrive with ONE cp.async.bulk per stage.
 //
 // CTA = one (b, z, 16 y-rows, full W) output slab of one parity class: MT = W/8 M-tiles of 128 rows, accumulators
-// MT x NPAD fp32 columns in TMEM.  Warps 0-3: halo producers (cp.async 16 B, zero-fill = padding), then epilogue
-// (tcgen05.ld -> scale/shift/LeakyReLU -> blocked store).  Warp 4: TMEM allocation + single-thread MMA issue.
+// MT x NPAD fp32 columns in TMEM.  Warps 0-3: halo producer (one thread issues the tensor copies, zero-fill = padding),
+// then epilogue (tcgen05.ld -> scale/shift/LeakyReLU -> blocked store).  Warp 4: TMEM allocation + single-thread MMA issue.
 // Pipeline: STAGES-deep ring of (halo chunk, weight chunk) with full/empty mbarriers; tcgen05.commit frees a slot.
 #include <cuda.h>   // CUtensorMap + the cuTensorMapEncodeTiled prototype (the entry point is resolved through the runtime: no -lcuda)
-#include <cstdlib>
 #include <cstring>
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -29,7 +28,6 @@
 namespace gb {
 
 constexpr int CT_THREADS = 160;       // 4 producer/epilogue warps + 1 MMA warp
-constexpr int CT_PRODUCERS = 128;
 constexpr int CT_BY = 16;             // y rows per CTA (16 core-matrix groups of 8 x positions = M 128)
 constexpr int CT_KCG = 2;             // channel groups (of 4) per stage = one K=8 TF32 MMA per tap and M-tile
 
@@ -59,18 +57,17 @@ struct ConvTParams {
 // so the hi*hi products and the 2^11-scaled cross terms keep separate accumulators (the tensor core's fp32 accumulator
 // truncates: a step's error scales with the partial sum it joins, and the cross terms would otherwise ride on the big one),
 // and the epilogue returns acc_hi + 2^-11 * acc_cross.  2 MMAs per K step instead of the 3 of a K-expanded split.
-// TMA: the halo of a channel group arrives as ONE cp.async.bulk.tensor (5-D tiled tensor map over [plane][cg][H][W][16 B], box
-// [1][1][PY][PX][16 B], out-of-bounds elements zero-filled = the convolution's padding) instead of PY*PX 16-byte cp.async
-// issued by 128 threads; each channel group then starts on a 128-byte boundary of shared memory (the LBO of the A descriptor
-// is that padded stride).
-template <int T, int NPAD, int MT, bool X2 = false, bool TMA = false>
+// Halo: a channel group arrives as ONE cp.async.bulk.tensor (5-D tiled tensor map over [plane][cg][H][W][16 B], box
+// [1][1][PY][PX][16 B], out-of-bounds elements zero-filled = the convolution's padding); each channel group starts on a
+// 128-byte boundary of shared memory (the LBO of the A descriptor is that padded stride).
+template <int T, int NPAD, int MT, bool X2 = false>
 struct ConvTCfg {
   static constexpr int W = 8 * MT;
   static constexpr int PY = CT_BY + T - 1, PX = W + T - 1;     // halo extent
   static constexpr int PARTS = X2 ? 2 : 1;
   static constexpr int NACC = PARTS * NPAD;                    // accumulator columns per M-tile = width of the B operand
   static constexpr int A_CG_BYTES = PY * PX * 16;              // one channel group of the halo
-  static constexpr int A_CG_STRIDE = TMA ? ((A_CG_BYTES + 127) / 128) * 128 : A_CG_BYTES;   // its pitch in shared memory = LBO of A
+  static constexpr int A_CG_STRIDE = ((A_CG_BYTES + 127) / 128) * 128;   // its pitch in shared memory = LBO of A
   static constexpr int A_BYTES = PARTS * CT_KCG * A_CG_STRIDE; // [part][channel group][halo]
   static constexpr int A_TX_BYTES = PARTS * CT_KCG * A_CG_BYTES;  // bytes the tensor copies of one stage deliver
   static constexpr int B_TAP_BYTES = 2 * (NACC / 8) * 128;     // one (y,x) tap: [2 kcore][NACC/8][8 rows][16 B]
@@ -93,8 +90,6 @@ struct ConvTCfg {
   static constexpr int S_PAIR = (112 * 1024) / STAGE_BYTES > 6 ? 6 : (112 * 1024) / STAGE_BYTES;
   static constexpr bool PAIR = TMEM_COLS <= 256 && S_PAIR >= 2;
   static constexpr int STAGES = PAIR ? S_PAIR : S_ALONE;
-  static constexpr int POS = PY * PX;
-  static constexpr int POS_PER_THREAD = (POS + CT_PRODUCERS - 1) / CT_PRODUCERS;
   static constexpr size_t SMEM = (size_t)STAGES * STAGE_BYTES + 256;
   static_assert(STAGES >= 2, "stage too large");
   static_assert(MT * NACC <= 512, "accumulators exceed TMEM");
@@ -117,11 +112,11 @@ struct ConvTCfg {
 //         N = 16 columns of which 8 are the output classes; the epilogue adds the bias (shift[0]), optionally applies
 //         the sigmoid, and writes the NCDHW fp32 volume directly.
 // OP: operand type: 0 = TF32 (fp32 storage), 1 = fp16, 2 = fp16 hi/lo split (X2, see ConvTCfg)
-template <int TZ, int T, int NPAD, int MT, int MODE, int OP, bool TMA>
+template <int TZ, int T, int NPAD, int MT, int MODE, int OP>
 __global__ void __launch_bounds__(CT_THREADS, 1)
 convt3d_s2_kernel(const ConvTParams p, const __grid_constant__ CUtensorMap tmap0, const __grid_constant__ CUtensorMap tmap1) {
   constexpr bool F16 = OP != 0, X2 = OP == 2;
-  using Cfg = ConvTCfg<T, NPAD, MT, X2, TMA>;
+  using Cfg = ConvTCfg<T, NPAD, MT, X2>;
   constexpr int NACC = Cfg::NACC;
   constexpr float LO_SCALE = 1.0f / 2048.0f;   // the cross-term accumulators hold 2^11 x their value
   constexpr bool PAR = MODE == 0, MERGE = MODE == 2, MERGE8 = MODE == 3, C1 = MODE == 4;
@@ -166,18 +161,11 @@ convt3d_s2_kernel(const ConvTParams p, const __grid_constant__ CUtensorMap tmap0
     return zi >= 0 && zi < p.D;
   };
   const int n_q = TZ * nchunk * Cfg::YS;
-  // Cluster of NCL CTAs along blockIdx.x (same parity class, hence the same weight sequence): every CTA fetches 1/NCL of each
-  // stage's weights and multicasts it to all of them, so the L2 serves the weights once per cluster instead of once per CTA.
-  // The CTAs then walk the SAME stage sequence in lockstep: a stage whose z-tap plane lies outside this CTA's volume is not
-  // skipped but walked without halo and without MMAs; a slot is free when every CTA's MMAs have released it.
-  const uint32_t ncl = cluster_nctarank(), crank = ncl > 1 ? cluster_ctarank() : 0;
-  const uint16_t cmask = (uint16_t)((1u << ncl) - 1);
 
   if (tid == 0) {
     for (int s = 0; s < Cfg::STAGES; ++s) {
-      mbar_init(&full[s], TMA ? 1 : CT_PRODUCERS + 1);  // cp.async path: 128 producer arrivals + the expect_tx arrival of the
-                                                        // weight copy; TMA path: the one expect_tx arrival (halo + weight bytes)
-      mbar_init(&empty[s], ncl);              // one tcgen05.commit per CTA of the cluster
+      mbar_init(&full[s], 1);   // the one expect_tx arrival (halo + weight bytes)
+      mbar_init(&empty[s], 1);  // the tcgen05.commit of the MMAs that read the slot
     }
     mbar_init(accum_full, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -190,119 +178,40 @@ convt3d_s2_kernel(const ConvTParams p, const __grid_constant__ CUtensorMap tmap0
   }
   tc_fence_before();
   __syncthreads();
-  if (ncl > 1) cluster_sync_all();   // every CTA's barriers exist before a peer's multicast can signal them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // weights of one stage: this CTA's slice, to every CTA of the cluster
-  auto load_weights = [&](uint8_t *dst, const float *wsrc, uint32_t bytes, uint64_t *bar) {
-    if (ncl == 1) {
-      bulk_g2s(dst, wsrc, bytes, bar);
-    } else {
-      const uint32_t slice = bytes / ncl;
-      bulk_g2s_multicast(dst + crank * slice, reinterpret_cast<const uint8_t *>(wsrc) + crank * slice, slice, bar, cmask);
-    }
-  };
 
   if (warp < 4) {
-    if constexpr (TMA) {
-      // ===================== producer: ONE thread issues the tensor copies of every stage ==========================
-      if (tid == 0) {
-        int it = 0;
-        for (int q = 0; q < n_q; ++q) {
-          int tz, kc, ys, bz, by, bx;
-          const bool valid = stage_of(q, tz, kc, ys, bz, by, bx);
-          if (!valid && ncl == 1) continue;
-          const int s = it % Cfg::STAGES, use = it / Cfg::STAGES;
-          ++it;
-          if (use > 0) mbar_wait(&empty[s], (use - 1) & 1);
-          uint8_t *sa = stages + (size_t)s * Cfg::STAGE_BYTES;
-          const int rows = (ys + 1) * Cfg::ROWS <= T ? Cfg::ROWS : T - ys * Cfg::ROWS;
-          const uint32_t wbytes = (uint32_t)(rows * T * Cfg::B_TAP_BYTES);
-          const float *wsrc = p.wpack + ((((size_t)par * TZ + tz) * nchunk + kc) * (size_t)(T * T * Cfg::B_TAP_BYTES / 4)) +
-                              (size_t)ys * Cfg::ROWS * T * (Cfg::B_TAP_BYTES / 4);
-          mbar_arrive_expect_tx(&full[s], wbytes + (valid ? (uint32_t)Cfg::A_TX_BYTES : 0u));
-          load_weights(sa + Cfg::A_BYTES, wsrc, wbytes, &full[s]);
-          if (!valid) continue;
-          const int zi = zj + bz - tz;
-          const int gy0 = y0 + by - (T - 1), gx0 = x0 + bx - (T - 1);
-#pragma unroll
-          for (int part = 0; part < Cfg::PARTS; ++part) {
-#pragma unroll
-            for (int c = 0; c < CT_KCG; ++c) {
-              int cg = kc * CT_KCG + c;
-              const CUtensorMap *tm = &tmap0;
-              if (cg >= p.cg0) { cg -= p.cg0; tm = &tmap1; }
-              tma_load_5d(sa + (part * CT_KCG + c) * Cfg::A_CG_STRIDE, tm, gx0, gy0, cg, (b * p.D + zi) * Cfg::PARTS + part, &full[s]);
-            }
-          }
-        }
-      }
-    } else {
-    // ===================== producers: halo (cp.async, zero-fill) + weights (one bulk copy per stage) ==========
-    // this thread's halo positions are the same for every stage: precompute (offset in the cg plane, halo row/col)
-    int hoff[Cfg::POS_PER_THREAD], hy[Cfg::POS_PER_THREAD], hx[Cfg::POS_PER_THREAD];
-#pragma unroll
-    for (int i = 0; i < Cfg::POS_PER_THREAD; ++i) {
-      const int idx = tid + i * CT_PRODUCERS;
-      hy[i] = idx / Cfg::PX;
-      hx[i] = idx - hy[i] * Cfg::PX;
-      hoff[i] = idx < Cfg::POS ? idx * 16 : -1;
-    }
-    constexpr int LAG = Cfg::STAGES - 1 < 2 ? 1 : 2;  // cp.async groups in flight before a stage is published
-    int it = 0;                                        // stages issued so far
-    auto publish = [&]() {  // after committing group `it`: group it - LAG has landed -> hand it to the async proxy
-      cp_async_commit();
-      if (it >= LAG) {
-        cp_async_wait<LAG>();
-        fence_proxy_async_smem();
-        mbar_arrive(&full[(it - LAG) % Cfg::STAGES]);
-      }
-      ++it;
-    };
-    for (int q = 0; q < n_q; ++q) {
-      int tz, kc, ys, bz, by, bx;
-      const bool valid = stage_of(q, tz, kc, ys, bz, by, bx);
-      if (!valid && ncl == 1) continue;
-      const int s = it % Cfg::STAGES, use = it / Cfg::STAGES;
-      if (use > 0) mbar_wait(&empty[s], (use - 1) & 1);
-      uint8_t *sa = stages + (size_t)s * Cfg::STAGE_BYTES;
-      if (tid == 0) {
+    // ===================== producer: ONE thread issues the tensor copies of every stage ==========================
+    if (tid == 0) {
+      int it = 0;
+      for (int q = 0; q < n_q; ++q) {
+        int tz, kc, ys, bz, by, bx;
+        if (!stage_of(q, tz, kc, ys, bz, by, bx)) continue;
+        const int s = it % Cfg::STAGES, use = it / Cfg::STAGES;
+        ++it;
+        if (use > 0) mbar_wait(&empty[s], (use - 1) & 1);
+        uint8_t *sa = stages + (size_t)s * Cfg::STAGE_BYTES;
         // weights of tap rows [ys*ROWS, ...) of this (class, z tap, K chunk): a contiguous slice of its T*T-tap block
         const int rows = (ys + 1) * Cfg::ROWS <= T ? Cfg::ROWS : T - ys * Cfg::ROWS;
-        const uint32_t bytes = (uint32_t)(rows * T * Cfg::B_TAP_BYTES);
+        const uint32_t wbytes = (uint32_t)(rows * T * Cfg::B_TAP_BYTES);
         const float *wsrc = p.wpack + ((((size_t)par * TZ + tz) * nchunk + kc) * (size_t)(T * T * Cfg::B_TAP_BYTES / 4)) +
                             (size_t)ys * Cfg::ROWS * T * (Cfg::B_TAP_BYTES / 4);
-        mbar_arrive_expect_tx(&full[s], bytes);
-        load_weights(sa + Cfg::A_BYTES, wsrc, bytes, &full[s]);
-      }
-      const int zi = zj + bz - tz;
-      const int gy0 = y0 + by - (T - 1), gx0 = x0 + bx - (T - 1);  // halo row hy holds input row gy0 + hy
-      if (valid) {
+        mbar_arrive_expect_tx(&full[s], wbytes + (uint32_t)Cfg::A_TX_BYTES);
+        bulk_g2s(sa + Cfg::A_BYTES, wsrc, wbytes, &full[s]);
+        const int zi = zj + bz - tz;
+        const int gy0 = y0 + by - (T - 1), gx0 = x0 + bx - (T - 1);  // halo row r holds input row gy0 + r
 #pragma unroll
-      for (int part = 0; part < Cfg::PARTS; ++part) {
+        for (int part = 0; part < Cfg::PARTS; ++part) {
 #pragma unroll
-        for (int c = 0; c < CT_KCG; ++c) {
-          int cg = kc * CT_KCG + c;
-          const float *src = p.src0;
-          int ncg = p.cg0;
-          if (cg >= p.cg0) { cg -= p.cg0; src = p.src1; ncg = p.cg1; }
-          // X2: [B*D][part][cg][H][W][16 B]
-          const float *plane = src + (((((size_t)b * p.D + zi) * Cfg::PARTS + part) * ncg + cg) * p.H) * (size_t)p.W * 4;
-#pragma unroll
-          for (int i = 0; i < Cfg::POS_PER_THREAD; ++i) {
-            if (hoff[i] < 0) continue;
-            const int gy = gy0 + hy[i], gx = gx0 + hx[i];
-            const bool ok = (gy >= 0) & (gy < p.H) & (gx >= 0) & (gx < p.W);
-            const float *g = ok ? plane + ((size_t)gy * p.W + gx) * 4 : plane;
-            cp_async16_zfill(sa + (part * CT_KCG + c) * Cfg::A_CG_STRIDE + hoff[i], g, ok);
+          for (int c = 0; c < CT_KCG; ++c) {
+            int cg = kc * CT_KCG + c;
+            const CUtensorMap *tm = &tmap0;
+            if (cg >= p.cg0) { cg -= p.cg0; tm = &tmap1; }
+            tma_load_5d(sa + (part * CT_KCG + c) * Cfg::A_CG_STRIDE, tm, gx0, gy0, cg, (b * p.D + zi) * Cfg::PARTS + part, &full[s]);
           }
         }
       }
-      }
-      publish();
-    }
-    for (int e = 0; e < LAG; ++e) publish();  // drain: empty groups push the last real ones through
-
     }
     // ===================== epilogue: TMEM -> registers -> act(acc*scale+shift) -> blocked global store =========
     mbar_wait(accum_full, 0);
@@ -422,13 +331,11 @@ convt3d_s2_kernel(const ConvTParams p, const __grid_constant__ CUtensorMap tmap0
     int it = 0;
     for (int q = 0; q < n_q; ++q) {
       int tz, kc, ys, bz, by, bx;
-      const bool valid = stage_of(q, tz, kc, ys, bz, by, bx);
-      if (!valid && ncl == 1) continue;
+      if (!stage_of(q, tz, kc, ys, bz, by, bx)) continue;
       const int s = it % Cfg::STAGES, use = it / Cfg::STAGES;
       ++it;
       mbar_wait(&full[s], use & 1);
       tc_fence_after();
-      if (valid) {
       const uint32_t sa = smem_u32(stages + (size_t)s * Cfg::STAGE_BYTES);
       const uint32_t sb = sa + Cfg::A_BYTES;
       const int ty0 = ys * Cfg::ROWS;
@@ -455,15 +362,11 @@ convt3d_s2_kernel(const ConvTParams p, const __grid_constant__ CUtensorMap tmap0
         }
       }
       first = false;
-      }
-      // frees the slot (in every CTA of the cluster) when the MMAs that read it are done (implies fence::before_thread_sync)
-      if (ncl == 1) umma_commit(&empty[s]);
-      else umma_commit_multicast(&empty[s], cmask);
+      umma_commit(&empty[s]);  // frees the slot when the MMAs that read it are done (implies fence::before_thread_sync)
     }
     umma_commit(accum_full);
   }
   __syncthreads();
-  if (ncl > 1) cluster_sync_all();   // no CTA leaves while a peer may still signal its barriers
   if (warp == 4) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(Cfg::TMEM_COLS) : "memory");
@@ -489,9 +392,9 @@ static EncodeTiledFn tmap_encoder() {
 }
 // blocked activations [planes][ncg][H][W][16 B] as a 5-D map of 4-byte elements (4, W, H, ncg, planes); box = one channel
 // group's halo (4, PX, PY, 1, 1); elements outside [0,W) x [0,H) are delivered as zeros
-static bool make_halo_tmap(CUtensorMap *m, const void *base, long long planes, int ncg, int H, int W, int PX, int PY) {
-  EncodeTiledFn enc = tmap_encoder();
-  if (!enc || !base || ncg <= 0) return false;
+static bool make_halo_tmap(EncodeTiledFn enc, CUtensorMap *m, const void *base, long long planes, int ncg, int H, int W, int PX,
+                           int PY) {
+  if (!base || ncg <= 0) return false;
   const cuuint64_t gdim[5] = {4, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)ncg, (cuuint64_t)planes};
   const cuuint64_t gstr[4] = {16, (cuuint64_t)W * 16, (cuuint64_t)H * W * 16, (cuuint64_t)ncg * H * W * 16};
   const cuuint32_t box[5] = {4, (cuuint32_t)PX, (cuuint32_t)PY, 1, 1};
@@ -499,31 +402,10 @@ static bool make_halo_tmap(CUtensorMap *m, const void *base, long long planes, i
   return enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT32, 5, const_cast<void *>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
              CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-// halo producer: tensor copies (default) or the cp.async path (GENRE_B200_CONV_TMA=0, or genre_b200_conv_set_tma(0))
-static int g_conv_tma = -1;
-static bool conv_use_tma() {
-  if (g_conv_tma < 0) {
-    const char *e = getenv("GENRE_B200_CONV_TMA");
-    g_conv_tma = (e && e[0] == '0') ? 0 : 1;
-  }
-  return g_conv_tma == 1 && tmap_encoder() != nullptr;
-}
-
-// CTAs per cluster sharing each stage's weights by multicast (GENRE_B200_CONV_CLUSTER, or genre_b200_conv_set_cluster): 1 = off
-static int g_conv_cluster = -1;
-static int conv_cluster() {
-  if (g_conv_cluster < 0) {
-    const char *e = getenv("GENRE_B200_CONV_CLUSTER");
-    const int v = e ? atoi(e) : 1;
-    g_conv_cluster = (v == 2 || v == 4 || v == 8) ? v : 1;
-  }
-  return g_conv_cluster;
-}
-
-template <int TZ, int T, int NPAD, int MT, int MODE, int OP, bool TMA>
+template <int TZ, int T, int NPAD, int MT, int MODE, int OP>
 static int launch_convt_variant(const ConvTParams &p, cudaStream_t st) {
-  using Cfg = ConvTCfg<T, NPAD, MT, OP == 2, TMA>;
-  auto kern = convt3d_s2_kernel<TZ, T, NPAD, MT, MODE, OP, TMA>;
+  using Cfg = ConvTCfg<T, NPAD, MT, OP == 2>;
+  auto kern = convt3d_s2_kernel<TZ, T, NPAD, MT, MODE, OP>;
   static bool configured[64] = {};
   int dev = 0;
   cudaGetDevice(&dev);
@@ -538,43 +420,19 @@ static int launch_convt_variant(const ConvTParams &p, cudaStream_t st) {
   ConvTParams q = p;
   q.xtiles = p.W / Cfg::W;
   if (q.xtiles < 1 || q.xtiles * Cfg::W != p.W) return fail_arg(GENRE_B200_EINVAL, "convt3d: W=%d is not a multiple of the %d-wide tile", p.W, Cfg::W);
+  const EncodeTiledFn enc = tmap_encoder();
+  if (!enc) return fail_arg(GENRE_B200_EINVAL, "convt3d: the CUDA driver does not provide cuTensorMapEncodeTiled");
   CUtensorMap tm0, tm1;
   memset(&tm0, 0, sizeof(tm0));
   memset(&tm1, 0, sizeof(tm1));
-  if (TMA) {
-    const long long planes = (long long)p.B * p.D * Cfg::PARTS;
-    if (!make_halo_tmap(&tm0, p.src0, planes, p.cg0, p.H, p.W, Cfg::PX, Cfg::PY))
-      return fail_arg(GENRE_B200_EINVAL, "convt3d: cuTensorMapEncodeTiled failed for the first operand");
-    if (p.cg1 > 0 && !make_halo_tmap(&tm1, p.src1, planes, p.cg1, p.H, p.W, Cfg::PX, Cfg::PY))
-      return fail_arg(GENRE_B200_EINVAL, "convt3d: cuTensorMapEncodeTiled failed for the second operand");
-  }
+  const long long planes = (long long)p.B * p.D * Cfg::PARTS;
+  if (!make_halo_tmap(enc, &tm0, p.src0, planes, p.cg0, p.H, p.W, Cfg::PX, Cfg::PY))
+    return fail_arg(GENRE_B200_EINVAL, "convt3d: cuTensorMapEncodeTiled failed for the first operand");
+  if (p.cg1 > 0 && !make_halo_tmap(enc, &tm1, p.src1, planes, p.cg1, p.H, p.W, Cfg::PX, Cfg::PY))
+    return fail_arg(GENRE_B200_EINVAL, "convt3d: cuTensorMapEncodeTiled failed for the second operand");
   dim3 grid((unsigned)(p.B * p.D * (p.H / CT_BY) * q.xtiles), MODE == 0 ? 8 : MODE == 2 ? 2 : 1);
-  int cl = conv_cluster();
-  while (cl > 1 && (grid.x % cl != 0 || (T * Cfg::B_TAP_BYTES) % (16 * cl) != 0)) cl /= 2;
-  if (cl > 1) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(CT_THREADS);
-    cfg.dynamicSmemBytes = Cfg::SMEM;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)cl;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (cudaLaunchKernelEx(&cfg, kern, q, tm0, tm1) != cudaSuccess) return check_launch("convt3d_s2 cluster launch");
-    return check_launch("convt3d_s2 kernel");
-  }
   kern<<<grid, CT_THREADS, Cfg::SMEM, st>>>(q, tm0, tm1);
   return check_launch("convt3d_s2 kernel");
-}
-
-template <int TZ, int T, int NPAD, int MT, int MODE, int OP>
-static int launch_convt_impl(const ConvTParams &p, cudaStream_t st) {
-  if (conv_use_tma()) return launch_convt_variant<TZ, T, NPAD, MT, MODE, OP, true>(p, st);
-  return launch_convt_variant<TZ, T, NPAD, MT, MODE, OP, false>(p, st);
 }
 
 static thread_local int g_conv_op = 0;  // operand type of the next launch (set by the C ABI entry points): 0 TF32, 1 fp16, 2 fp16 hi/lo
@@ -586,13 +444,13 @@ static int launch_convt_x2(const ConvTParams &p, cudaStream_t st) {
   } else if constexpr (MT * 2 * NPAD > 512) {
     return launch_convt_x2<TZ, T, NPAD, MT / 2, MODE>(p, st);
   } else {
-    return launch_convt_impl<TZ, T, NPAD, MT, MODE, 2>(p, st);
+    return launch_convt_variant<TZ, T, NPAD, MT, MODE, 2>(p, st);
   }
 }
 template <int TZ, int T, int NPAD, int MT, int MODE>
 static int launch_convt_op(const ConvTParams &p, cudaStream_t st) {
   if (g_conv_op == 2) return launch_convt_x2<TZ, T, NPAD, MT, MODE>(p, st);
-  return g_conv_op == 1 ? launch_convt_impl<TZ, T, NPAD, MT, MODE, 1>(p, st) : launch_convt_impl<TZ, T, NPAD, MT, MODE, 0>(p, st);
+  return g_conv_op == 1 ? launch_convt_variant<TZ, T, NPAD, MT, MODE, 1>(p, st) : launch_convt_variant<TZ, T, NPAD, MT, MODE, 0>(p, st);
 }
 template <int T, int NPAD, int MT, bool PAR>
 static int launch_convt(const ConvTParams &p, cudaStream_t st) {
@@ -606,7 +464,7 @@ template <int MT>
 static int launch_convt_c1(const ConvTParams &p, cudaStream_t st) {
   if (g_conv_op == 2)   // not routed (ops_conv.convt_c1_tc): the exact FP32-pipe stencil serves the fp32-accurate modes
     return fail_arg(GENRE_B200_EINVAL, "convt_c1_tc: the fp16 hi/lo operand mode is not supported for the 1-channel layer");
-  return g_conv_op == 1 ? launch_convt_impl<3, 3, 16, MT, 4, 1>(p, st) : launch_convt_impl<3, 3, 16, MT, 4, 0>(p, st);
+  return g_conv_op == 1 ? launch_convt_variant<3, 3, 16, MT, 4, 1>(p, st) : launch_convt_variant<3, 3, 16, MT, 4, 0>(p, st);
 }
 template <int T, int NPAD, int MT>
 static int launch_conv_merged8(const ConvTParams &p, cudaStream_t st) {
@@ -616,22 +474,6 @@ static int launch_conv_merged8(const ConvTParams &p, cudaStream_t st) {
 }  // namespace gb
 
 using namespace gb;
-
-// Select the halo producer of the convolution kernels: 1 = cp.async.bulk.tensor (TMA, default), 0 = 16-byte cp.async by 128
-// threads.  Returns the previous setting.  Process-wide; meant for A/B timing and for testing both producers in one process.
-extern "C" int genre_b200_conv_set_tma(int enable) {
-  const int prev = conv_use_tma() ? 1 : 0;
-  g_conv_tma = enable ? 1 : 0;
-  return prev;
-}
-
-// CTAs per thread-block cluster of the convolution kernels (1, 2, 4 or 8): the CTAs of a cluster share every stage's weights
-// through multicast bulk copies.  Returns the previous setting.  Process-wide; for A/B timing and tests.
-extern "C" int genre_b200_conv_set_cluster(int ctas) {
-  const int prev = conv_cluster();
-  g_conv_cluster = (ctas == 2 || ctas == 4 || ctas == 8) ? ctas : 1;
-  return prev;
-}
 
 // ConvTranspose3d(kernel K in {4, 8}, stride 2, padding K/2 - 1) forward on channel-blocked activations.
 //   src0 [B*D][cg0][H][W][4], src1 [B*D][cg1][H][W][4] or NULL: the two halves of the channel concatenation

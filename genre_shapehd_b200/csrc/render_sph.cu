@@ -13,12 +13,13 @@
 // shuffle product-scan and crosses 32-sample chunks through a register carry.  Only the [N,S,S] map
 // is written.  Sample positions are formed in fp64 from the fp64 direction table exactly like the
 // numpy code, then rounded to fp32, so they equal the reference's registered `grid` buffer.
-#include <cstdlib>
 #include "common.cuh"
 
 namespace gb {
 
 constexpr int RS_THREADS = 256;  // 8 rays per CTA
+// resident CTAs per SM of the skipping renderer: bounds its registers (48, with 64 B of spills) and sizes its one-wave grid
+constexpr int RS_OCC = 5;
 
 struct Taps {
   int base;        // linear index of corner (x0, y0, z0); may be out of range, see masks
@@ -269,9 +270,8 @@ render_occupancy128_kernel(const float *__restrict__ vox, unsigned *__restrict__
   }
 }
 
-// OCC: resident CTAs per SM the register allocation is bounded for (5: 48 registers with 64 B of spills; 4: 64, none)
-template <bool PRE, int OCC>
-__global__ void __launch_bounds__(RS_THREADS, OCC)
+template <bool PRE>
+__global__ void __launch_bounds__(RS_THREADS, RS_OCC)
 render_spherical_forward_skip_kernel(const float *__restrict__ vox, int R, const double *__restrict__ dirs, int S, int Z,
                                      const float *__restrict__ depth_weight, const unsigned *__restrict__ occ,
                                      float *__restrict__ out, const VoxPre pre) {
@@ -636,25 +636,17 @@ extern "C" int genre_b200_render_spherical_forward_skip(const float *vox, int64_
   }
   if (int rc = check_launch("render_spherical occupancy kernel")) return rc;
   const int ngroups = (sph_res * sph_res + 3) / 4;
-  // one wave of resident CTAs over the whole batch (OCC per SM, 148 SMs), warps stride over the ray groups
-  static int occ = 0;
-  if (!occ) {
-    const char *e = getenv("GENRE_B200_RENDER_OCC");   // tuning knob (profiles/): 4 or 5
-    occ = (e && atoi(e) == 4) ? 4 : 5;
-  }
-  int ctas = (int)((148 * occ) / N);
+  // one wave of resident CTAs over the whole batch (RS_OCC per SM, 148 SMs), warps stride over the ray groups
+  int ctas = (int)((148 * RS_OCC) / N);
   const int max_ctas = (ngroups + RS_THREADS / 32 - 1) / (RS_THREADS / 32);
   if (ctas > max_ctas) ctas = max_ctas;
   if (ctas < 1) ctas = 1;
   dim3 rg((unsigned)ctas, (unsigned)N);
-#define GB_RS_LAUNCH(PRE_, OCC_)                                                                                              \
-  render_spherical_forward_skip_kernel<PRE_, OCC_><<<rg, RS_THREADS, 0, st>>>(vox, res, dirs, sph_res, z_res, depth_weight, \
-                                                                              (const unsigned *)workspace, out, pre)
-  if (use_pre) {
-    if (occ == 4) GB_RS_LAUNCH(true, 4); else GB_RS_LAUNCH(true, 5);
-  } else {
-    if (occ == 4) GB_RS_LAUNCH(false, 4); else GB_RS_LAUNCH(false, 5);
-  }
-#undef GB_RS_LAUNCH
+  if (use_pre)
+    render_spherical_forward_skip_kernel<true><<<rg, RS_THREADS, 0, st>>>(vox, res, dirs, sph_res, z_res, depth_weight,
+                                                                         (const unsigned *)workspace, out, pre);
+  else
+    render_spherical_forward_skip_kernel<false><<<rg, RS_THREADS, 0, st>>>(vox, res, dirs, sph_res, z_res, depth_weight,
+                                                                          (const unsigned *)workspace, out, pre);
   return check_launch("render_spherical forward kernel (empty-space skipping)");
 }

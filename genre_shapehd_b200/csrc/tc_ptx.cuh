@@ -1,5 +1,5 @@
-// tc_ptx.cuh — the PTX wrappers shared by the tcgen05 kernels (convt3d.cu, convflat.cu): mbarriers, cp.async / bulk / tensor
-// copies, UMMA descriptors and instructions, TMEM loads.
+// tc_ptx.cuh — the PTX wrappers shared by the tcgen05 kernels (convt3d.cu, convflat.cu): mbarriers, bulk / tensor copies,
+// UMMA descriptors and instructions, TMEM loads.
 #pragma once
 #include <cuda.h>   // CUtensorMap
 #include "common.cuh"
@@ -34,13 +34,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
     if (spin > (1u << 26)) asm volatile("trap;");
   }
 }
-__device__ __forceinline__ void cp_async16_zfill(void *sdst, const void *gsrc, bool valid) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(sdst)), "l"(gsrc), "r"(valid ? 16 : 0)
-               : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void bulk_g2s(void *sdst, const void *gsrc, uint32_t bytes, uint64_t *bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                    smem_u32(sdst)),
@@ -54,7 +47,6 @@ __device__ __forceinline__ void tma_load_5d(void *sdst, const CUtensorMap *tmap,
       ::"r"(smem_u32(sdst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(0), "r"(x), "r"(y), "r"(cg), "r"(plane), "r"(smem_u32(bar))
       : "memory");
 }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
@@ -90,33 +82,6 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
 }
 __device__ __forceinline__ void umma_commit(uint64_t *bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// ---- thread-block clusters: rank / size, cluster-wide barrier, multicast forms of the bulk copy and of the MMA commit ----------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t cluster_nctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// the bytes land at the same shared-memory offset of every CTA in `mask`, each of whose mbarriers (same offset) gets the complete_tx
-__device__ __forceinline__ void bulk_g2s_multicast(void *sdst, const void *gsrc, uint32_t bytes, uint64_t *bar, uint16_t mask) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-                   smem_u32(sdst)),
-               "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)), "h"(mask)
-               : "memory");
-}
-// one arrival on the mbarrier at this offset in every CTA of `mask` when the MMAs issued so far are done
-__device__ __forceinline__ void umma_commit_multicast(uint64_t *bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(mask)
                : "memory");
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {

@@ -8,7 +8,7 @@ namespace gb {
 // ------------------------------------------------------------------------------------------------
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-static size_t counters_words(int64_t n_maps, size_t nt) { return (size_t)n_maps * nt + (size_t)n_maps + (size_t)n_maps + 1; }
+static size_t counters_words(int64_t n_maps, size_t nt) { return (size_t)n_maps * nt + (size_t)n_maps; }
 static size_t counters_bytes(int64_t n_maps, size_t nt) { return align_up(counters_words(n_maps, nt) * 4, 256); }
 
 size_t vox_workspace_bytes(int64_t n_maps, int64_t P, int res) {
@@ -25,7 +25,6 @@ bool vox_carve(void *ws, size_t ws_bytes, int64_t n_maps, int64_t P, int res, Vo
   char *p = (char *)ws;
   out->counts = (unsigned *)p;
   out->ovf_count = out->counts + (size_t)n_maps * nt;
-  out->sync = out->ovf_count + (size_t)n_maps;
   p += counters_bytes(n_maps, nt);
   out->buckets = (uint2 *)p;
   p += align_up((size_t)n_maps * nt * VOX_BUCKET * 8, 256);

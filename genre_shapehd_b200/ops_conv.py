@@ -65,8 +65,6 @@ PRECISION = os.environ.get("GENRE_B200_CONV_PRECISION", "exact")
 EXACT_IMPL = os.environ.get("GENRE_B200_CONV_EXACT_IMPL", "f16x2")
 # k=8 ConvTranspose3d with Cout <= 20 (Unet_3D.dec5): merge the four (y,x) parity classes into one N=80 MMA stream
 MERGE_PARITIES = os.environ.get("GENRE_B200_CONV_MERGE", "1") != "0"
-# Unet_3D.enc1 (4x space-to-depth form): z class on blockIdx.y (N = 80, two CTAs per SM) instead of all 8 classes in N = 160
-S4D_SPLIT_Z = os.environ.get("GENRE_B200_S4D_SPLIT_Z", "0") != "0"   # measured: 0.88 vs 0.80 ms, so off
 
 
 # With torch.backends.cudnn.allow_tf32 off the caller asks for fp32 convolutions: the kernels then run the 3xTF32 scheme
@@ -1235,7 +1233,9 @@ def conv3d(x, m, bn=None, slope=None):
         if aff is None:
             return None
         g, b, cout = _group(), x.shape[0], m.out_channels
-        split_z = S4D_SPLIT_Z or _x2()     # f16x2 doubles the accumulator columns: 8 classes x 20 x 2 = 320 > 256, 4 classes fit
+        # f16x2 doubles the accumulator columns: 8 classes x 20 x 2 = 320 > 256, so the z class moves to blockIdx.y (N = 80).
+        # The other modes keep all 8 classes in N = 160 (the split form measured 0.88 vs 0.80 ms for them).
+        split_z = _x2()
         wpack = _pack(m, ("k8s2_s4d", 20, g, split_z), lambda wt: pack_conv_k8s2_s4d_weights(wt, 20, g, split_z),
                       2 if split_z else 1)
         if _x2_direct(x):

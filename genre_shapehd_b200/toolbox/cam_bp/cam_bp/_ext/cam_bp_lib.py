@@ -50,7 +50,7 @@ def back_projection_forward(depth, camdist, fl, voxel, cnt, shift=False):
     _lib.call("genre_b200_cam_bp_forward", depth.data_ptr(), n, c, h, w, *depth.stride(),
               fl.data_ptr(), *fl.stride(), camdist.data_ptr(), *camdist.stride(),
               voxel.data_ptr(), cnt.data_ptr() if cnt is not None else None, res,
-              (_lib.FLAG_SHIFT_TDF if shift else 0) | _lib.CAM_BP_FLAGS, ws.data_ptr(), nbytes, _lib.stream_ptr(depth))
+              _lib.FLAG_SHIFT_TDF if shift else 0, ws.data_ptr(), nbytes, _lib.stream_ptr(depth))
     return 1
 
 

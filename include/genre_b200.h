@@ -35,9 +35,6 @@ extern "C" {
 
 /* flags for the projection entry points */
 #define GENRE_B200_FLAG_SHIFT_TDF 1u /* fuse Camera_back_projection_layer.shift_tdf: 1 - R*tdf */
-#define GENRE_B200_FLAG_OVERLAP 2u  /* cam_bp_forward, experimental: project and splat overlapped in ONE kernel (interleaved block
-                                      order, per-map completion counters).  Measured on B200: slower than back to back (75.9 vs
-                                      68.0 us at batch 32), so off by default; see DESIGN.md 4.1 */
 
 const char *genre_b200_last_error(void);
 /* library/ABI version: major*1000 + minor */
@@ -58,6 +55,7 @@ int genre_b200_version(void);
  *             with    SHIFT: 1 - R*mean on hit voxels, 1 - R*(1/R) elsewhere
  *   cnt     [N, C, R, R, R] dense or NULL; if given, the per-voxel point count as fp32 (what the
  *             reference keeps on ctx for backward, cam_back_projection.py:28)
+ *   flags   0 or GENRE_B200_FLAG_SHIFT_TDF; any other bit is rejected with GENRE_B200_EINVAL
  *   workspace: genre_b200_voxelize_workspace_bytes(N*C, H*W, R) bytes, 16-byte aligned
  * ------------------------------------------------------------------------------------------- */
 size_t genre_b200_voxelize_workspace_bytes(int64_t n_maps, int64_t pixels_per_map, int res);
@@ -377,16 +375,6 @@ int genre_b200_sph_bp_forward_fused(const float *sph, int64_t N, int64_t C, int6
  * (`torch.clamp(proj_depth / 50, 1e-5, 1 - 1e-5)` + torch.cat, genre_full_model.py:126-127). */
 int genre_b200_scale_clamp_strided(const float *src, int64_t maps, int64_t n, float scale, float lo, float hi,
                                    float *dst, int64_t dst_map_stride, void *stream);
-
-/* Halo producer of the convolution kernels: 1 = cp.async.bulk.tensor over a 5-D tiled tensor map (default), 0 = cp.async by 128
- * threads (round 1).  Returns the previous setting; process-wide (A/B timing, tests).  Env: GENRE_B200_CONV_TMA. */
-int genre_b200_conv_set_tma(int enable);
-
-/* CTAs per thread-block cluster of the convolution kernels of csrc/convt3d.cu (1 = no clusters, 2, 4 or 8): the CTAs of a cluster
- * walk the same weight sequence, each fetches 1/n of every stage's weights and multicasts it to all of them (cp.async.bulk
- * .multicast::cluster), and a pipeline slot is released by a multicast tcgen05.commit.  Default: GENRE_B200_CONV_CLUSTER or 1.
- * Returns the previous setting.  Process-wide. */
-int genre_b200_conv_set_cluster(int ctas);
 
 /* blocked fp32 [BD][cg4][H][W][4] -> blocked fp16 [BD][(cg4+1)/2][H][W][8], channel padding zero-filled: turns the
  * fp32 output of one tensor-core layer into the fp16 operand of the next without going through NCDHW */

@@ -31,7 +31,7 @@ def test_library_exports_every_declared_symbol():
 
 def test_version_and_error_string():
     lib = _lib.load()
-    assert lib.genre_b200_version() >= 1000
+    assert lib.genre_b200_version() >= 2000
     # argument errors are reported without touching the device
     rc = lib.genre_b200_nnd_forward(None, None, 1, 1, 1, None, None, None, None, None)
     assert rc == -1
@@ -92,6 +92,9 @@ def _d(v=4096):
     (lambda L: L.genre_b200_conv_k8s2_wgrad(_d(), _d(), 1, 3, 20, 2, 16, 16, _d(), _d(), 1 << 30, None), -1, b"Cin"),
     # fused glue
     (lambda L: L.genre_b200_render_spherical_forward_pre(_d(), 1, 16, _d(), 8, 16, _d(), 50.0, 1.0, 0.0, _d(), None), -1, b"clamp"),
+    # projection flags: only GENRE_B200_FLAG_SHIFT_TDF is defined, any other bit is refused rather than ignored
+    (lambda L: L.genre_b200_cam_bp_forward(_d(), 1, 1, 16, 16, 256, 256, 16, 1, _d(), 1, 1, _d(), 1, 1, _d(), None, 16, 2, _d(),
+                                           1 << 30, None), -1, b"flag"),
 ])
 def test_conv_and_layout_entry_points_validate_before_launching(call, code, needle):
     """every unsupported shape / misaligned buffer is an argument error with a message, reported without touching a GPU"""

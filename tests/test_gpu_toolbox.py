@@ -666,21 +666,3 @@ def test_nnd_full_size_symmetry_and_minimality():
     probe = b[:, torch.randint(0, 16384, (256,), device=DEV, generator=gen)]          # [4,256,3]
     dp = ((a.unsqueeze(2) - probe.unsqueeze(1)) ** 2).sum(-1).min(-1).values
     assert (d1 <= dp + 1e-7).all()
-
-
-def test_cam_bp_overlap_kernel_equals_the_two_kernel_path():
-    """GENRE_B200_FLAG_OVERLAP (project and splat interleaved in one kernel, per-map completion counters; off by default because it
-    measured slower) produces bit-identical volumes: same records, same integer accumulation"""
-    from genre_shapehd_b200.synth import bench_depth_batch
-    x = torch.from_numpy(bench_depth_batch(12)).to(DEV)
-    fl = torch.full((12, 1), 418.3, device=DEV)
-    cd = torch.full((12, 1), 2.2, device=DEV)
-    outs = []
-    for flags in (_lib.FLAG_SHIFT_TDF, _lib.FLAG_SHIFT_TDF | _lib.FLAG_OVERLAP):
-        ws, nbytes = _lib.workspace_for(12, 256 * 256, 128, DEV)
-        tdf = torch.empty(12, 1, 128, 128, 128, device=DEV)
-        cnt = torch.empty_like(tdf)
-        _lib.call("genre_b200_cam_bp_forward", x.data_ptr(), 12, 1, 256, 256, *x.stride(), fl.data_ptr(), *fl.stride(), cd.data_ptr(),
-                  *cd.stride(), tdf.data_ptr(), cnt.data_ptr(), 128, flags, ws.data_ptr(), nbytes, _lib.stream_ptr(x))
-        outs.append((tdf, cnt))
-    assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
