@@ -72,6 +72,9 @@ _SIGNATURES = {
     "genre_b200_cam_bp_stage_project": [_ptr] + [_i64] * 8 + [_ptr, _i64, _i64, _ptr, _i64, _i64, _int, _ptr, _size,
                                                              _ptr],
     "genre_b200_voxelize_stage_splat": [_i64, _i64, _int, _ptr, _ptr, _f32, _f32, _f32, _ptr, _size, _ptr],
+    "genre_b200_iso_surface_count": [_ptr, _i64, _int, _int, _int, _f32, _ptr, _size, _ptr, _ptr],
+    "genre_b200_iso_surface_emit": [_ptr, _i64, _int, _int, _int, _f32] + [_f32] * 6 + [_ptr, _ptr, _ptr, _ptr, _ptr, _size,
+                                                                                         _ptr],
 }
 
 # every symbol include/genre_b200.h declares (tests check the library exports all of them)
@@ -79,7 +82,8 @@ EXPORTED_SYMBOLS = sorted(list(_SIGNATURES) + [
     "genre_b200_last_error", "genre_b200_version", "genre_b200_voxelize_workspace_bytes",
     "genre_b200_convt_c1_wgrad_workspace_bytes", "genre_b200_conv_k8s2_wgrad_workspace_bytes",
     "genre_b200_bn_workspace_bytes", "genre_b200_render_spherical_workspace_bytes",
-    "genre_b200_voxel_surface_workspace_bytes", "genre_b200_convflat_positions", "genre_b200_skinny_gemm_workspace_bytes"])
+    "genre_b200_voxel_surface_workspace_bytes", "genre_b200_convflat_positions", "genre_b200_skinny_gemm_workspace_bytes",
+    "genre_b200_iso_surface_workspace_bytes"])
 
 _lib = None
 launch_count = 0  # kernels of this library enqueued through the binding (bench.py reports it as gpu_launches)
@@ -97,6 +101,7 @@ _LAUNCHES = {
     "genre_b200_bn_act_train_forward": 3, "genre_b200_bn_act_train_backward": 2, "genre_b200_conv_k8s2_wgrad": 2, "genre_b200_convt_c1_wgrad": 2, "genre_b200_convt_c1_dgrad": 1,
     "genre_b200_blocked_split3": 1, "genre_b200_blocked_split2_f16": 1, "genre_b200_voxel_surface": 2, "genre_b200_convt_c1_col2im_forward": 1, "genre_b200_skinny_gemm": 2, "genre_b200_convflat_pack": 1, "genre_b200_convflat_forward": 1, "genre_b200_convt_c1_tc_forward": 1, "genre_b200_blocked_f32_to_f16": 1,
     "genre_b200_convt3d_s2_merged_forward": 1, "genre_b200_conv3d_k8s2_s4d_forward": 1, "genre_b200_ncdhw_to_blocked": 1, "genre_b200_blocked_to_ncdhw": 1,
+    "genre_b200_iso_surface_count": 3, "genre_b200_iso_surface_emit": 1,
 }
 
 
@@ -133,6 +138,8 @@ def load():
     lib.genre_b200_convflat_positions.argtypes = [_i64, _int, _int, _int, ctypes.POINTER(ctypes.c_int)]
     lib.genre_b200_voxel_surface_workspace_bytes.restype = _size
     lib.genre_b200_voxel_surface_workspace_bytes.argtypes = [_i64, _int]
+    lib.genre_b200_iso_surface_workspace_bytes.restype = _size
+    lib.genre_b200_iso_surface_workspace_bytes.argtypes = [_i64, _int, _int, _int]
     _lib = lib
     return lib
 

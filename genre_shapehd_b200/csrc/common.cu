@@ -29,4 +29,4 @@ const char *last_error() { return g_err; }
 }  // namespace gb
 
 extern "C" const char *genre_b200_last_error(void) { return gb::last_error(); }
-extern "C" int genre_b200_version(void) { return 2000; }
+extern "C" int genre_b200_version(void) { return 2001; }

@@ -407,6 +407,41 @@ size_t genre_b200_voxel_surface_workspace_bytes(int64_t N, int res);
 int genre_b200_voxel_surface(const float *vox, int64_t N, int res, int iterations, int transpose_flip, float *out,
                              void *workspace, size_t workspace_bytes, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Batched marching cubes (the mesh export of the reference's visualiser).  Replaces the per-sample CPU
+ * call of Visualizer._save_iso_obj (visualize/visualizer.py:153-166: skimage.measure.marching_cubes_lewiner
+ * in a process pool) for a whole batch on the device.  The case table is genre_shapehd_b200/csrc/mc_table.h,
+ * generated from a rule by gen_mc_table.py: ambiguous faces cut off each in-corner, cube-interior
+ * ambiguities are not resolved (no MC33), so in ambiguous cells the triangles and the topology can differ
+ * from Lewiner's; the vertices are the same iso-crossings of grid edges.
+ *
+ *   vol     [N, D, H, W] dense fp32; 1 <= N <= 65535, D, H >= 2, 2 <= W <= 256, 3*D*H*W and 5*(D-1)(H-1)(W-1)
+ *           within int32.  A voxel is inside when value > level (NaN: outside).
+ *   workspace: genre_b200_iso_surface_workspace_bytes(N, D, H, W) bytes, 16-byte aligned, caller-owned
+ *           (1 bit per voxel + 16 bytes per z row); emit reads what count wrote there, so the two calls must
+ *           share the workspace, the volume and the level, in stream order.
+ *
+ * _count: per-sample totals[N][2] int64 = (vertices, triangles), written on the device (the caller reads
+ *           them back to size the mesh buffers).  3 kernels.
+ * _emit:  bases[N][2] int64 = where each sample's vertices / triangles start in verts / faces (usually the
+ *           exclusive prefix sum of totals); verts [sum V, 3] fp32, faces [sum F, 3] int32 with indices local
+ *           to the sample, values [sum V] fp32 or NULL.  1 kernel.
+ *   Order (a contract: the output is deterministic and equal bit for bit to the oracle): one vertex per
+ *   crossed grid edge p -> p + e_a, sorted by the C-order index of p, then by a; faces sorted by cell
+ *   (C order), then by triangle index in the table.  Each operation rounds once:
+ *       t       = (level - f(p)) / (f(p + e_a) - f(p))
+ *       coord_a = (p_a + t) * s_a + o_a,   coord_b = p_b * s_b + o_b   (b != a)
+ *   with (s, o) = (sx, ox) for array axis 0 (D), (sy, oy) for axis 1 (H), (sz, oz) for axis 2 (W);
+ *   values = max(f(p), f(p + e_a)).  Triangle normals (right hand) point from the > level side to the
+ *   <= level side.
+ * ------------------------------------------------------------------------------------------- */
+size_t genre_b200_iso_surface_workspace_bytes(int64_t N, int D, int H, int W);
+int genre_b200_iso_surface_count(const float *vol, int64_t N, int D, int H, int W, float level, void *workspace,
+                                 size_t workspace_bytes, int64_t *totals, void *stream);
+int genre_b200_iso_surface_emit(const float *vol, int64_t N, int D, int H, int W, float level, float sx, float sy,
+                                float sz, float ox, float oy, float oz, const int64_t *bases, float *verts, int *faces,
+                                float *values, void *workspace, size_t workspace_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
